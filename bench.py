@@ -456,6 +456,8 @@ def run_ours(args, rank: int, world_size: int, local_rank: int):
     launches = dw.counters().kernelLaunches - launches0
     counters = dw.counters()
     stage_ms = dw.stage_ms()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dw, sc, counters.bodyCapacity)
 
     # ---- e2e: public API with host buffers, H2D + D2H inside the timed region ----
     idx = np.array([b.index for b in sc.bodies[1:]], dtype=np.int32)
@@ -573,6 +575,29 @@ def run_ours(args, rank: int, world_size: int, local_rank: int):
         dist.destroy_process_group()
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+DUMP_FIELDS = (("body_origin", "origin"), ("body_rotation", "rot"), ("body_linear_velocity", "linearVelocity"),
+               ("body_angular_velocity", "angularVelocity"))
+
+
+def dump_outputs(out_dir: str, dw, sc, body_capacity: int) -> None:
+    """The body state a caller of the timed step reads back after its last step: body origin (what s2Body_GetPosition and
+    s2World_GetBodyTransforms return), rotation (sin, cos), linear and angular velocity, one row per body of the scene in
+    creation order (the static ground first), as float32 .npy files; body_index.npy (float64) names each row's body.
+    36 bytes per body: above 64 MB a fixed, seeded sample of the bodies is written, in creation order."""
+    n = len(sc.bodies)
+    keep = np.arange(n)
+    per_body = 4 * 7 + 8
+    if n * per_body > DUMP_BUDGET_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BUDGET_BYTES // per_body, replace=False))
+    rows = dw.download_all_bodies(body_capacity)
+    rows = rows[np.array([sc.bodies[k].index for k in keep], dtype=np.int64)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "body_index.npy"), keep.astype(np.float64))
+    for name, field in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(rows[field], dtype=np.float32))
+
+
 def cpu_baseline(args) -> dict:
     """Bounded sample of the same workload on the unmodified reference, one host core."""
     from oracle import ref
@@ -618,6 +643,8 @@ def main():
     ap.add_argument("--no-colour-probe", action="store_true")
     ap.add_argument("--probe-base", type=int, default=2600, help="pyramid base of the per-colour kernel roofline probe")
     ap.add_argument("--cpu-steps", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the body state of the last one to DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 

@@ -7,7 +7,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from oracle import ref as refmod
+import lockstep
 from solver2d_b200 import capi, device, scenes
 from solver2d_b200.capi import Capsule, Circle, Vec2, default_body_def, default_mouse_def, default_revolute_def, default_shape_def
 
@@ -196,48 +196,102 @@ def _script(s: Session, phase: int):
         s.body("again", capi.DYNAMIC_BODY, (0.0, 12.0), ("box", 0.4, 0.4))
 
 
+QUERY_BOXES = (((-7.0, -0.5), (0.0, 4.0)), ((-30.0, -3.0), (30.0, 30.0)), ((7.0, 3.0), (10.0, 7.0)))
+TEST_POINTS = ((0.1, 0.5), (-3.0, 1.0), (8.0, 4.0))
+
+
+def _draw_entries(log) -> np.ndarray:
+    """A draw log as sorted strings (primitive and the exact bits of its numbers)."""
+    return np.array(sorted(name + ":" + ",".join(float(v).hex() for v in vals) for name, vals in log))
+
+
+def _session_readback(lib, s: Session, phase: int) -> dict:
+    """What the scripted-session test compares after a phase."""
+    out = {f"p{phase}_state": s.state(), f"p{phase}_contacts": np.array(lib.s2World_GetStatistics(s.world).contactCount)}
+    for k, (lo, hi) in enumerate(QUERY_BOXES):
+        out[f"p{phase}_query{k}"] = np.array(_query(lib, s.world, lo, hi), dtype=np.int64).reshape(-1, 2)
+    out[f"p{phase}_test_point"] = np.array([[lib.s2Shape_TestPoint(s.shapes[name], Vec2(*pt)) for pt in TEST_POINTS]
+                                            for name in sorted(s.shapes)[:12]], dtype=bool)
+    out[f"p{phase}_draw"] = _draw_entries(_draw_log(lib, s.world))
+    return out
+
+
+def _reference_session(solver):
+    def run(R):
+        sr = Session(R, solver)
+        out = {}
+        for phase in range(4):
+            _script(sr, phase)
+            out.update(lockstep.pack_keys(lockstep.reference_steps(R, sr.world, 45, DT), prefix=f"p{phase}_"))
+            out.update(_session_readback(R, sr, phase))
+        R.s2DestroyWorld(sr.world)
+        return out
+    return run
+
+
 @pytest.mark.parametrize("solver", ["TGS_Soft", "PGS_NGS_Block"])
-def test_scripted_session_matches_reference(reference, dev, solver):
-    from test_e2e_gpu import _ref_pair_table
-    R = reference
+def test_scripted_session_matches_reference(dev, solver):
+    ref = lockstep.Run(f"session_{solver.lower()}")
     P = capi.Solver2D(device.LIB_PATH)
-    sr, sp = Session(R, solver), Session(P, solver)
+    sp = Session(P, solver)
     dw = None
     for phase in range(4):
-        _script(sr, phase)
         _script(sp, phase)
         if dw is None:
             dw = device.DeviceWorld.attach(dev, sp.world)
             dw.set_schedule(device.SCHEDULE_WAVEFRONT)
         for step in range(45):
-            R.step_collide(sr.world)
-            keys, *_ = _ref_pair_table(R, sr.world)
-            dw.set_contact_order(keys)
-            R.step_solve(sr.world, DT, 4, 2, True)
-            R.step_finalize(sr.world)
+            dw.set_contact_order(ref.keys(step, prefix=f"p{phase}_"))
             P.step(sp.world, DT, 4, 2, True)
-        a, b = sr.state(), sp.state()
+        got = _session_readback(P, sp, phase)
+        a, b = ref[f"p{phase}_state"], got[f"p{phase}_state"]
         assert np.array_equal(a, b), f"phase {phase}: bodies differ, max {np.abs(a - b).max()}"
-        assert R.s2World_GetStatistics(sr.world).contactCount == P.s2World_GetStatistics(sp.world).contactCount
+        assert int(ref[f"p{phase}_contacts"]) == int(got[f"p{phase}_contacts"])
         # queries and debug draw read the same state back
-        for lo, hi in (((-7.0, -0.5), (0.0, 4.0)), ((-30.0, -3.0), (30.0, 30.0)), ((7.0, 3.0), (10.0, 7.0))):
-            assert _query(R, sr.world, lo, hi) == _query(P, sp.world, lo, hi)
-        for name in sorted(sr.shapes)[:12]:
-            for pt in ((0.1, 0.5), (-3.0, 1.0), (8.0, 4.0)):
-                assert R.s2Shape_TestPoint(sr.shapes[name], Vec2(*pt)) == P.s2Shape_TestPoint(sp.shapes[name], Vec2(*pt))
-        dr, dp = _draw_log(R, sr.world), _draw_log(P, sp.world)
+        for k in range(len(QUERY_BOXES)):
+            assert np.array_equal(ref[f"p{phase}_query{k}"], got[f"p{phase}_query{k}"])
+        assert np.array_equal(ref[f"p{phase}_test_point"], got[f"p{phase}_test_point"])
+        dr, dp = ref[f"p{phase}_draw"], got[f"p{phase}_draw"]
         assert len(dr) == len(dp) and len(dr) > 20
-        assert sorted(dr) == sorted(dp), "s2World_Draw output differs"
-    R.s2DestroyWorld(sr.world)
+        assert np.array_equal(dr, dp), "s2World_Draw output differs"
     P.s2DestroyWorld(sp.world)
 
 
-def test_edge_cases_match_reference(reference, dev):
+def _edge_case_session(lib):
+    s = Session(lib, "TGS_Soft")
+    s.body("ground", capi.STATIC_BODY, (0.0, -1.0), ("box", 40.0, 1.0))
+    for i in range(8):
+        s.body(f"a{i}", capi.DYNAMIC_BODY, (-3.0 + 0.9 * i, 0.6 + 0.05 * i), ("box", 0.4, 0.4))
+    return s
+
+
+def _grow(s):
+    for k in range(300):
+        s.body(f"g{k}", capi.DYNAMIC_BODY, (-15.0 + 0.11 * k, 3.0 + 1.1 * (k % 7)), ("circle", 0.3) if k % 2 else ("box", 0.3, 0.3))
+
+
+# (steps, dt, velocity iterations, relax iterations) of each run; the pools grow before the last one
+EDGE_RUNS = ((20, DT, 4, 2), (3, 0.0, 4, 2), (10, DT, 4, 0), (40, DT, 4, 2))
+
+
+def _reference_edge_cases(R):
+    sr = _edge_case_session(R)
+    out = {}
+    for k, (steps, dt, vel, pos) in enumerate(EDGE_RUNS):
+        if k == len(EDGE_RUNS) - 1:
+            _grow(sr)
+        out.update(lockstep.pack_keys(lockstep.reference_steps(R, sr.world, steps, dt, vel, pos), prefix=f"r{k}_"))
+        out[f"r{k}_state"] = sr.state()
+    out["body_count"] = np.array(R.s2World_GetStatistics(sr.world).bodyCount)
+    R.s2DestroyWorld(sr.world)
+    return out
+
+
+def test_edge_cases_match_reference(dev):
     """Empty world, a paused step (dt = 0: reference src/world.c:176-183 still runs the solver with inv_dt = 0), growth of
     every pool after the world has been stepped (device columns re-allocated, solver graph re-captured), and a step with
     zero relax iterations — all against the reference, reference order imposed."""
-    from test_e2e_gpu import _ref_pair_table
-    R = reference
+    ref = lockstep.Run("edge_cases")
     P = capi.Solver2D(device.LIB_PATH)
     # 1. an empty world steps (and reads back) without complaint
     we = P.create_world("TGS_Soft")
@@ -245,74 +299,67 @@ def test_edge_cases_match_reference(reference, dev):
     assert P.s2World_GetStatistics(we).bodyCount == 0
     P.s2DestroyWorld(we)
 
-    sr, sp = Session(R, "TGS_Soft"), Session(P, "TGS_Soft")
-    for s in (sr, sp):
-        s.body("ground", capi.STATIC_BODY, (0.0, -1.0), ("box", 40.0, 1.0))
-        for i in range(8):
-            s.body(f"a{i}", capi.DYNAMIC_BODY, (-3.0 + 0.9 * i, 0.6 + 0.05 * i), ("box", 0.4, 0.4))
+    sp = _edge_case_session(P)
     dw = device.DeviceWorld.attach(dev, sp.world)
     dw.set_schedule(device.SCHEDULE_WAVEFRONT)
-
-    def run(steps, dt, vel, pos):
-        for _ in range(steps):
-            R.step_collide(sr.world)
-            keys, *_ = _ref_pair_table(R, sr.world)
-            dw.set_contact_order(keys)
-            R.step_solve(sr.world, dt, vel, pos, True)
-            R.step_finalize(sr.world)
+    # 20 steps, 3 paused, 10 without relax iterations, then (2.) pools grow well past their initial capacity after stepping
+    for k, (steps, dt, vel, pos) in enumerate(EDGE_RUNS):
+        if k == len(EDGE_RUNS) - 1:
+            _grow(sp)
+        for step in range(steps):
+            dw.set_contact_order(ref.keys(step, prefix=f"r{k}_"))
             P.step(sp.world, dt, vel, pos, True)
-        a, b = sr.state(), sp.state()
-        assert np.array_equal(a, b), f"max {np.abs(a - b).max()}"
-
-    run(20, DT, 4, 2)
-    run(3, 0.0, 4, 2)      # paused
-    run(10, DT, 4, 0)      # no relax iterations
-    # 2. pools grow well past their initial capacity after stepping
-    for s in (sr, sp):
-        for k in range(300):
-            s.body(f"g{k}", capi.DYNAMIC_BODY, (-15.0 + 0.11 * k, 3.0 + 1.1 * (k % 7)), ("circle", 0.3) if k % 2 else ("box", 0.3, 0.3))
-    run(40, DT, 4, 2)
-    assert P.s2World_GetStatistics(sp.world).bodyCount == R.s2World_GetStatistics(sr.world).bodyCount == 309
-    R.s2DestroyWorld(sr.world)
+        a, b = ref[f"r{k}_state"], sp.state()
+        assert np.array_equal(a, b), f"run {k}: max {np.abs(a - b).max()}"
+    assert P.s2World_GetStatistics(sp.world).bodyCount == int(ref["body_count"]) == 309
     P.s2DestroyWorld(sp.world)
 
 
-def test_body_recreated_in_the_same_slot_at_the_same_place(reference, dev):
+def _recreate_script(lib):
+    """Rest a stack, then replace the second box of the middle column by a new one at the same place, at rest; returns
+    the contact count and the new box's height over the next 30 steps."""
+    sc = scenes.vertical_stack(lib, "TGS_Soft", count=4, columns=3)
+    for _ in range(40):
+        sc.step(DT, 4, 2, True)
+    victim = sc.bodies[1 + 4 + 1]
+    pos = lib.s2Body_GetPosition(victim)
+    lib.s2DestroyBody(victim)
+    bd = default_body_def()
+    bd.type = capi.DYNAMIC_BODY
+    bd.position = Vec2(pos.x, pos.y)
+    bid = lib.s2CreateBody(sc.world, C.byref(bd))
+    sd = default_shape_def()
+    box = lib.s2MakeSquare(0.5)
+    lib.s2CreatePolygonShape(bid, C.byref(sd), C.byref(box))
+    sc.bodies[1 + 4 + 1] = bid
+    counts, ys = [], []
+    for _ in range(30):
+        sc.step(DT, 4, 2, True)
+        counts.append(lib.s2World_GetStatistics(sc.world).contactCount)
+        ys.append(lib.s2Body_GetPosition(bid).y)
+    sc.destroy()
+    return counts, ys
+
+
+def _reference_recreated(R):
+    counts, ys = _recreate_script(R)
+    return dict(counts=np.array(counts, dtype=np.int64), ys=np.array(ys, dtype=np.float64))
+
+
+def test_body_recreated_in_the_same_slot_at_the_same_place(dev):
     """A resting box is destroyed and a new one is created where it stood: the new body re-uses the body and shape slots
     (and the proxy id) of the old one, so the contact table still holds the OLD shape's pairs under the same keys when the
     next pair pass runs. The pass has to drop those and report the pairs of the new shape in the same pass (the reference
     removes the keys on destroy and re-creates the contacts on its next update); otherwise the new box has no contacts
     until it leaves its fat AABB and sinks into its neighbours."""
-    R = reference
-    P = capi.Solver2D(device.LIB_PATH)
-
-    def script(lib):
-        sc = scenes.vertical_stack(lib, "TGS_Soft", count=4, columns=3)
-        for _ in range(40):
-            sc.step(DT, 4, 2, True)
-        # replace the second box of the middle column by a new one at the same place, at rest
-        victim = sc.bodies[1 + 4 + 1]
-        pos = lib.s2Body_GetPosition(victim)
-        lib.s2DestroyBody(victim)
-        bd = default_body_def()
-        bd.type = capi.DYNAMIC_BODY
-        bd.position = Vec2(pos.x, pos.y)
-        bid = lib.s2CreateBody(sc.world, C.byref(bd))
-        sd = default_shape_def()
-        box = lib.s2MakeSquare(0.5)
-        lib.s2CreatePolygonShape(bid, C.byref(sd), C.byref(box))
-        sc.bodies[1 + 4 + 1] = bid
-        counts, ys = [], []
-        for _ in range(30):
-            sc.step(DT, 4, 2, True)
-            counts.append(lib.s2World_GetStatistics(sc.world).contactCount)
-            ys.append(lib.s2Body_GetPosition(bid).y)
-        return sc, counts, ys
-
-    sr, cr, yr = script(R)
-    sp, cp, yp = script(P)
+    ref = lockstep.Run("body_recreated")
+    cr, yr = ref["counts"].tolist(), ref["ys"].tolist()
+    cp, yp = _recreate_script(capi.Solver2D(device.LIB_PATH))
     assert cp == cr, f"contact counts after re-creating the body: device {cp[:6]}... reference {cr[:6]}..."
     assert max(abs(a - b) for a, b in zip(yr, yp)) < 2e-3, "the re-created box does not rest where the reference's does"
     assert min(yp) > yr[0] - 0.02, "the re-created box sank into its neighbour"
-    sr.destroy()
-    sp.destroy()
+
+
+# what tests/golden/make_lockstep.py records from the reference: name -> run(R) -> arrays
+REFERENCE_RUNS = {f"session_{s.lower()}": _reference_session(s) for s in ("TGS_Soft", "PGS_NGS_Block")}
+REFERENCE_RUNS.update(edge_cases=_reference_edge_cases, body_recreated=_reference_recreated)

@@ -1,6 +1,7 @@
 """CPU: the product library loads without a GPU, exports every symbol the headers declare, and its host-side geometry and
 narrow-phase code (csrc/shared/s2_collide.h — the SAME source the CUDA narrow-phase kernel compiles) is bit-identical to
-the unmodified reference on seeded inputs. No world is created here: s2CreateWorld needs a CUDA device by design."""
+the unmodified reference on seeded inputs (its outputs recorded in tests/golden/host_vectors_ref.npz by
+tests/golden/make_host_vectors.py). No world is created here: s2CreateWorld needs a CUDA device by design."""
 import ctypes as C
 import re
 
@@ -44,88 +45,101 @@ def test_row_struct_sizes_match_numpy_mirrors():
     assert out[4] == C.sizeof(device.StepContext) and out[5] == C.sizeof(device.Counters)
 
 
-def _same_bytes(a, b):
-    return bytes(a) == bytes(b)
+GOLDEN = os.path.join(ROOT, "tests", "golden", "host_vectors_ref.npz")
 
 
-def _poly_eq(p, q):
-    n = p.count
-    return (p.count == q.count and p.radius == q.radius
-            and all(p.vertices[i].x == q.vertices[i].x and p.vertices[i].y == q.vertices[i].y for i in range(n))
-            and all(p.normals[i].x == q.normals[i].x and p.normals[i].y == q.normals[i].y for i in range(n)))
+def _poly(p) -> np.ndarray:
+    """A polygon as the compared fields: count, radius, then its vertices and normals (unused slots zero)."""
+    out = np.zeros(2 + 32, dtype=np.float32)
+    out[0], out[1] = p.count, p.radius
+    for i in range(p.count):
+        out[2 + 2 * i:4 + 2 * i] = (p.vertices[i].x, p.vertices[i].y)
+        out[18 + 2 * i:20 + 2 * i] = (p.normals[i].x, p.normals[i].y)
+    return out
 
 
-def test_polygon_factories_and_mass_match_reference(reference, product):
-    R, P = reference, product
+def _raw(struct) -> np.ndarray:
+    return np.frombuffer(bytes(struct), dtype=np.uint8).copy()
+
+
+def box_with_radius(L, hx, hy):
+    """What s2MakeRoundedBox(hx, hy, 0.1) stands for: a box polygon with a 0.1 radius."""
+    p = L.s2MakeBox(hx, hy)
+    p.radius = 0.1
+    return p
+
+
+def polygon_factory_outputs(L, rounded_box=None) -> np.ndarray:
+    """Box / offset box / rounded box / capsule factories, their mass data and a polygon AABB on seeded inputs, as bytes.
+    The rounded box comes from L's s2MakeRoundedBox unless `rounded_box(L, hx, hy)` builds it."""
     rng = np.random.default_rng(7)
+    out = []
     for _ in range(50):
         hx, hy = rng.uniform(0.05, 3.0, 2)
         ang = rng.uniform(-3, 3)
         c = capi.Vec2(*rng.uniform(-2, 2, 2))
-        assert _poly_eq(R.s2MakeBox(hx, hy), P.s2MakeBox(hx, hy))
-        a, b = R.s2MakeOffsetBox(hx, hy, c, ang), P.s2MakeOffsetBox(hx, hy, c, ang)
-        assert _poly_eq(a, b)
+        out.append(_poly(L.s2MakeBox(hx, hy)).view(np.uint8))
+        a = L.s2MakeOffsetBox(hx, hy, c, ang)
+        out.append(_poly(a).view(np.uint8))
         for dens in (1.0, 20.0):
-            ma, mb = R.s2ComputePolygonMass(C.byref(a), dens), P.s2ComputePolygonMass(C.byref(b), dens)
-            assert _same_bytes(ma, mb)
-        rb = P.s2MakeRoundedBox(hx, hy, 0.1)
-        ra = R.s2MakeBox(hx, hy)
-        ra.radius = 0.1
-        assert _same_bytes(R.s2ComputePolygonMass(C.byref(ra), 2.0), P.s2ComputePolygonMass(C.byref(rb), 2.0))
+            out.append(_raw(L.s2ComputePolygonMass(C.byref(a), dens)))
+        rb = rounded_box(L, hx, hy) if rounded_box is not None else L.s2MakeRoundedBox(hx, hy, 0.1)
+        out.append(_raw(L.s2ComputePolygonMass(C.byref(rb), 2.0)))
         p1, p2 = capi.Vec2(*rng.uniform(-1, 1, 2)), capi.Vec2(*rng.uniform(1.5, 3, 2))
-        assert _poly_eq(R.s2MakeCapsule(p1, p2, 0.3), P.s2MakeCapsule(p1, p2, 0.3))
+        out.append(_poly(L.s2MakeCapsule(p1, p2, 0.3)).view(np.uint8))
         cap = capi.Capsule(p1, p2, 0.3)
-        assert _same_bytes(R.s2ComputeCapsuleMass(C.byref(cap), 1.5), P.s2ComputeCapsuleMass(C.byref(cap), 1.5))
+        out.append(_raw(L.s2ComputeCapsuleMass(C.byref(cap), 1.5)))
         xf = capi.Transform(c, capi.Rot(np.float32(np.sin(ang)), np.float32(np.cos(ang))))
-        assert _same_bytes(R.s2ComputePolygonAABB(C.byref(a), xf), P.s2ComputePolygonAABB(C.byref(b), xf))
+        out.append(_raw(L.s2ComputePolygonAABB(C.byref(a), xf)))
+    return np.concatenate(out)
 
 
-def test_hull_matches_reference(reference, product):
-    R, P = reference, product
+def hull_outputs(L) -> np.ndarray:
+    """Quickhull on seeded point sets (welded / collinear inputs among them) and the polygon made from each hull."""
     rng = np.random.default_rng(11)
+    out = []
     for trial in range(200):
         n = int(rng.integers(3, 9))
         pts = (capi.Vec2 * n)(*[capi.Vec2(*rng.uniform(-1.5, 1.5, 2)) for _ in range(n)])
         if trial % 5 == 0:  # welded / collinear inputs
             pts[1] = capi.Vec2(pts[0].x + 0.001, pts[0].y)
-        ha, hb = R.s2ComputeHull(pts, n), P.s2ComputeHull(pts, n)
-        assert ha.count == hb.count
-        for i in range(ha.count):
-            assert ha.points[i].x == hb.points[i].x and ha.points[i].y == hb.points[i].y
-        if ha.count >= 3:
-            assert _poly_eq(R.s2MakePolygon(C.byref(ha)), P.s2MakePolygon(C.byref(hb)))
+        h = L.s2ComputeHull(pts, n)
+        row = np.zeros(1 + 16, dtype=np.float32)
+        row[0] = h.count
+        for i in range(h.count):
+            row[1 + 2 * i:3 + 2 * i] = (h.points[i].x, h.points[i].y)
+        out.append(row)
+        out.append(_poly(L.s2MakePolygon(C.byref(h))) if h.count >= 3 else np.zeros(34, np.float32))
+    return np.concatenate(out)
 
 
-def _manifold_eq(a, b):
-    if a.pointCount != b.pointCount:
-        return False
-    if a.pointCount == 0:
-        return True
-    if (a.normal.x, a.normal.y) != (b.normal.x, b.normal.y):
-        return False
-    for i in range(a.pointCount):
-        pa, pb = a.points[i], b.points[i]
-        if (pa.localAnchorA.x, pa.localAnchorA.y, pa.localAnchorB.x, pa.localAnchorB.y, pa.separation, pa.id) != \
-                (pb.localAnchorA.x, pb.localAnchorA.y, pb.localAnchorB.x, pb.localAnchorB.y, pb.separation, pb.id):
-            return False
-    return True
+def _manifold(m) -> np.ndarray:
+    """pointCount, then (normal, per point: anchors, separation, id) when it has points; the compared fields only."""
+    out = np.zeros(3 + 2 * 6, dtype=np.float32)
+    out[0] = m.pointCount
+    if m.pointCount:
+        out[1:3] = (m.normal.x, m.normal.y)
+        for i in range(m.pointCount):
+            p = m.points[i]
+            out[3 + 6 * i:8 + 6 * i] = (p.localAnchorA.x, p.localAnchorA.y, p.localAnchorB.x, p.localAnchorB.y, p.separation)
+            out[8 + 6 * i:9 + 6 * i] = np.array([p.id], dtype=np.int32).view(np.float32)
+    return out
 
 
-def test_manifold_functions_match_reference_bitwise(reference, product):
+def manifold_outputs(L) -> np.ndarray:
     """All nine shape-pair manifold functions (reference src/contact.c:139-154) on random near-contact configurations,
-    with the GJK cache carried over several perturbed calls as a persistent contact does."""
-    R, P = reference, product
+    with the GJK cache carried over several perturbed calls as a persistent contact does: (trials, 3, 9 + 5, 15)."""
     rng = np.random.default_rng(2024)
 
     def xf(x, y, ang):
         return capi.Transform(capi.Vec2(x, y), capi.Rot(np.float32(np.sin(ang)), np.float32(np.cos(ang))))
 
-    hits = 0
+    out = np.zeros((400, 3, 14, 15), dtype=np.float32)
     for trial in range(400):
-        boxA = R.s2MakeBox(*rng.uniform(0.3, 1.2, 2))
+        boxA = L.s2MakeBox(*rng.uniform(0.3, 1.2, 2))
         pts = (capi.Vec2 * 6)(*[capi.Vec2(*rng.uniform(-0.8, 0.8, 2)) for _ in range(6)])
-        hull = R.s2ComputeHull(pts, 6)
-        polyB = R.s2MakePolygon(C.byref(hull)) if hull.count >= 3 else R.s2MakeBox(0.5, 0.4)
+        hull = L.s2ComputeHull(pts, 6)
+        polyB = L.s2MakePolygon(C.byref(hull)) if hull.count >= 3 else L.s2MakeBox(0.5, 0.4)
         polyB.radius = 0.05 if trial % 3 == 0 else 0.0
         circ = capi.Circle(capi.Vec2(*rng.uniform(-0.2, 0.2, 2)), float(rng.uniform(0.2, 0.6)))
         circ2 = capi.Circle(capi.Vec2(0.0, 0.0), float(rng.uniform(0.2, 0.6)))
@@ -134,28 +148,52 @@ def test_manifold_functions_match_reference_bitwise(reference, product):
         seg = capi.Segment(capi.Vec2(-1.0, 0.0), capi.Vec2(1.0, float(rng.uniform(-0.3, 0.3))))
         d = rng.uniform(0.6, 1.9)
         th = rng.uniform(0, 2 * np.pi)
-        cacheR = [capi.DistanceCache() for _ in range(5)]
-        cacheP = [capi.DistanceCache() for _ in range(5)]
+        cache = [capi.DistanceCache() for _ in range(5)]
         for it in range(3):  # persistent cache across slightly moved poses
             A = xf(*rng.uniform(-0.01, 0.01, 2), rng.uniform(-0.02, 0.02) + 0.3 * trial)
             B = xf(d * np.cos(th) + rng.uniform(-0.01, 0.01), d * np.sin(th) + rng.uniform(-0.01, 0.01), rng.uniform(-3, 3) if it == 0 else 0.1 * it)
-            pairs = [
-                (R.s2CollideCircles(C.byref(circ), A, C.byref(circ2), B), P.s2CollideCircles(C.byref(circ), A, C.byref(circ2), B)),
-                (R.s2CollideCapsuleAndCircle(C.byref(cap), A, C.byref(circ), B), P.s2CollideCapsuleAndCircle(C.byref(cap), A, C.byref(circ), B)),
-                (R.s2CollideSegmentAndCircle(C.byref(seg), A, C.byref(circ), B), P.s2CollideSegmentAndCircle(C.byref(seg), A, C.byref(circ), B)),
-                (R.s2CollidePolygonAndCircle(C.byref(boxA), A, C.byref(circ), B), P.s2CollidePolygonAndCircle(C.byref(boxA), A, C.byref(circ), B)),
-                (R.s2CollidePolygons(C.byref(boxA), A, C.byref(polyB), B, C.byref(cacheR[0])), P.s2CollidePolygons(C.byref(boxA), A, C.byref(polyB), B, C.byref(cacheP[0]))),
-                (R.s2CollideCapsules(C.byref(cap), A, C.byref(cap2), B, C.byref(cacheR[1])), P.s2CollideCapsules(C.byref(cap), A, C.byref(cap2), B, C.byref(cacheP[1]))),
-                (R.s2CollidePolygonAndCapsule(C.byref(boxA), A, C.byref(cap), B, C.byref(cacheR[2])), P.s2CollidePolygonAndCapsule(C.byref(boxA), A, C.byref(cap), B, C.byref(cacheP[2]))),
-                (R.s2CollideSegmentAndCapsule(C.byref(seg), A, C.byref(cap), B, C.byref(cacheR[3])), P.s2CollideSegmentAndCapsule(C.byref(seg), A, C.byref(cap), B, C.byref(cacheP[3]))),
-                (R.s2CollideSegmentAndPolygon(C.byref(seg), A, C.byref(polyB), B, C.byref(cacheR[4])), P.s2CollideSegmentAndPolygon(C.byref(seg), A, C.byref(polyB), B, C.byref(cacheP[4]))),
+            ms = [
+                L.s2CollideCircles(C.byref(circ), A, C.byref(circ2), B),
+                L.s2CollideCapsuleAndCircle(C.byref(cap), A, C.byref(circ), B),
+                L.s2CollideSegmentAndCircle(C.byref(seg), A, C.byref(circ), B),
+                L.s2CollidePolygonAndCircle(C.byref(boxA), A, C.byref(circ), B),
+                L.s2CollidePolygons(C.byref(boxA), A, C.byref(polyB), B, C.byref(cache[0])),
+                L.s2CollideCapsules(C.byref(cap), A, C.byref(cap2), B, C.byref(cache[1])),
+                L.s2CollidePolygonAndCapsule(C.byref(boxA), A, C.byref(cap), B, C.byref(cache[2])),
+                L.s2CollideSegmentAndCapsule(C.byref(seg), A, C.byref(cap), B, C.byref(cache[3])),
+                L.s2CollideSegmentAndPolygon(C.byref(seg), A, C.byref(polyB), B, C.byref(cache[4])),
             ]
-            for k, (mr, mp) in enumerate(pairs):
-                assert _manifold_eq(mr, mp), f"trial {trial} iter {it} function {k}"
-                hits += mr.pointCount > 0
-            for cr, cp in zip(cacheR, cacheP):
-                assert cr.count == cp.count and bytes(cr.indexA) == bytes(cp.indexA) and bytes(cr.indexB) == bytes(cp.indexB)
-    assert hits > 1500  # the sweep actually produced contacts
+            for k, m in enumerate(ms):
+                out[trial, it, k] = _manifold(m)
+            for k, cc in enumerate(cache):
+                out[trial, it, 9 + k, 0] = cc.count
+                out[trial, it, 9 + k, 1:4] = list(bytes(cc.indexA))[:3]
+                out[trial, it, 9 + k, 4:7] = list(bytes(cc.indexB))[:3]
+    return out
+
+
+def _golden(key):
+    return np.load(GOLDEN)[key]
+
+
+def test_polygon_factories_and_mass_match_reference(product):
+    want = _golden("polygon_factories")
+    got = polygon_factory_outputs(product)
+    assert got.shape == want.shape and np.array_equal(got, want)
+
+
+def test_hull_matches_reference(product):
+    want = _golden("hull")
+    got = hull_outputs(product)
+    assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
+
+
+def test_manifold_functions_match_reference_bitwise(product):
+    want = _golden("manifolds")
+    got = manifold_outputs(product)
+    bad = np.nonzero((got.view(np.uint32) != want.view(np.uint32)).any(axis=-1))
+    assert len(bad[0]) == 0, f"first mismatch: trial {bad[0][0]} iter {bad[1][0]} function/cache {bad[2][0]}"
+    assert (want[:, :, :9, 0] > 0).sum() > 1500  # the sweep actually produced contacts
 
 
 def _atan2_inputs(n, seed):

@@ -14,17 +14,20 @@ Instead every step is checked on its own against the reference pipeline fed with
     compare                       ->  bodies (position, rotation, velocities, origin) and manifold / joint impulses, bitwise
 
 The reference world is advanced with the oracle's result (bodies and warm-start impulses), so its broad phase, contact pool
-and manifold ids evolve exactly as if the reference had solved in the device's order."""
+and manifold ids evolve exactly as if the reference had solved in the device's order. tests/golden/make_multistep.py runs
+that pipeline and stores, for every step, a SHA-256 digest of what it produced (tests/golden/multistep/); the tests compute
+the same digest from what the device produced and compare, step by step."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
-from helpers import bit_equal, body_rows_from_ref, contact_rows_from_ref, joint_rows_from_ref
-from oracle import port
-from oracle import ref as refmod
 from solver2d_b200 import capi, device, scenes
 
 pytestmark = pytest.mark.gpu
 DT = 1.0 / 60.0
+MULTISTEP_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "multistep")
 
 
 @pytest.fixture(scope="module")
@@ -32,188 +35,154 @@ def product():
     return capi.Solver2D(device.LIB_PATH)
 
 
-def _load_bodies_into_ref(R, wid, rows):
-    """Device body rows -> the reference world's bodies (state fields only; mass data and flags are construction-time)."""
-    F = refmod.BODY_F
-    bf, bi = R.bodies(wid)
-    n = min(len(rows), bf.shape[0])
-    valid = bi[:n, 0] == 1
-    for name, col, width in (("origin", F["origin"], 2), ("position", F["position"], 2), ("rot", F["rot"], 2),
-                             ("linearVelocity", F["v"], 2)):
-        bf[:n, col:col + width][valid] = rows[name][:n][valid]
-    bf[:n, F["w"]][valid] = rows["angularVelocity"][:n][valid]
-    bf[:n, F["dp"]:F["dp"] + 2][valid] = 0.0
-    bf[:n, F["force"]:F["force"] + 2][valid] = rows["force"][:n][valid]
-    bf[:n, F["torque"]][valid] = rows["torque"][:n][valid]
-    R.load_body_state(wid, bf)
+def step_digest(shape_a, shape_b, point_count, body_valid, bodies, normal, tangent, joint_valid, joints) -> bytes:
+    """Digest of one step's compared results: the contact table (shape pairs in key order, point counts), every valid body
+    (position, rotation, velocities, origin), the impulses of the live manifolds and of the valid joints."""
+    h = hashlib.sha256()
+
+    def put(a, dtype):
+        h.update(np.ascontiguousarray(a, dtype=dtype).tobytes())
+    for a in (shape_a, shape_b, point_count):
+        put(a, np.int32)
+    for name in ("position", "rot", "linearVelocity", "origin", "angularVelocity"):
+        put(bodies[name][body_valid], np.float32)
+    live = np.asarray(point_count) > 0
+    put(normal[live], np.float32)
+    put(tangent[live], np.float32)
+    for name in ("impulse", "motorImpulse", "lowerImpulse", "upperImpulse"):
+        put(joints[name][joint_valid], np.float32)
+    return h.digest()
 
 
-def _run(R, P, dev, recipe, solver, steps, vel, pos, kw, min_replays=0, setup=None):
-    O = port.load()
-    sr = recipe(R, solver, **kw)
+def device_step_digest(dw) -> bytes:
+    c = dw.counters()
+    got = dw.download_contacts(c.contactCount + 64)
+    post = dw.download_all_bodies(c.bodyCapacity)
+    joints = dw.download_joints(c.jointCapacity)
+    return step_digest(got["shapeA"], got["shapeB"], got["pointCount"], (post["flags"] & 1) == 1, post,
+                       got["points"]["normalImpulse"], got["points"]["tangentImpulse"], (joints["flags"] & 1) == 1, joints)
+
+
+def start(dev, P, recipe, solver, kw, setup=None):
+    """The product's scene, pushed to the device now (s2World_Step would do it): the first step is checked like any other."""
     sp = recipe(P, solver, **kw)
-    # push the freshly built scene to the device now (s2World_Step would do it): the first step is checked like any other
     dev.lib.s2World_Flush.restype = None
     dev.lib.s2World_Flush.argtypes = [capi.WorldId]
     dev.lib.s2World_Flush(sp.world)
     dw = device.DeviceWorld.attach(dev, sp.world)
     if setup is not None:
         setup(dw)
-    ctx = device.make_context(solver, DT, vel, pos, True)
-    worst = {}
+    return sp, dw
+
+
+def _run(P, dev, name, min_replays=0):
+    recipe, solver, steps, vel, pos, kw, setup = CASES[name]
+    want = np.load(os.path.join(MULTISTEP_DIR, name + ".npy"))
+    assert want.shape == (steps, 32)
+    sp, dw = start(dev, P, recipe, solver, kw, setup)
     for step in range(steps):
-        cap = R.capacities(sr.world)["bodyCap"]
-        pre = dw.download_all_bodies(cap)
-        _load_bodies_into_ref(R, sr.world, pre)
-        R.step_collide(sr.world)
-
         sp.step(DT, vel, pos, True)
-
-        bodies = body_rows_from_ref(*R.bodies(sr.world))
-        cf, ci = R.contacts(sr.world)
-        rows_slot, slots = contact_rows_from_ref(cf, ci)
-        keys = (np.minimum(rows_slot["shapeA"], rows_slot["shapeB"]).astype(np.uint64) << np.uint64(32)) | \
-            np.maximum(rows_slot["shapeA"], rows_slot["shapeB"]).astype(np.uint64)
-        perm = np.argsort(keys, kind="stable")
-        rows_key = rows_slot[perm]
-        joints = joint_rows_from_ref(*R.joints(sr.world))
-
-        got_contacts = dw.download_contacts(len(rows_key) + 64)
-        assert len(got_contacts) == len(rows_key), f"step {step}: contact tables differ in size"
-        assert np.array_equal(got_contacts["shapeA"], rows_key["shapeA"]) and np.array_equal(got_contacts["shapeB"], rows_key["shapeB"]), \
-            f"step {step}: pair set or (A, B) order differs"
-        assert np.array_equal(got_contacts["pointCount"], rows_key["pointCount"]), f"step {step}: manifold point counts differ"
-
-        order, sizes = dw.solve_order(len(rows_key) + len(joints) + 16, max_groups=200000)
-        ob, oc, oj = O.solve(capi.SOLVER[solver], bodies, rows_key, joints, ctx, order=order)
-
-        # advance the reference world with the oracle's result
-        F = refmod.BODY_F
-        bf, bi = R.bodies(sr.world)
-        valid = bi[:, 0] == 1
-        bf[:, F["position"]:F["position"] + 2][valid] = ob["position"][valid]
-        bf[:, F["rot"]:F["rot"] + 2][valid] = ob["rot"][valid]
-        bf[:, F["v"]:F["v"] + 2][valid] = ob["linearVelocity"][valid]
-        bf[:, F["w"]][valid] = ob["angularVelocity"][valid]
-        bf[:, F["dp"]:F["dp"] + 2][valid] = 0.0
-        R.load_body_state(sr.world, bf)
-        imp = np.zeros((cf.shape[0], 4), dtype=np.float32)
-        imp[slots[perm], 0] = oc["points"]["normalImpulse"][:, 0]
-        imp[slots[perm], 1] = oc["points"]["tangentImpulse"][:, 0]
-        imp[slots[perm], 2] = oc["points"]["normalImpulse"][:, 1]
-        imp[slots[perm], 3] = oc["points"]["tangentImpulse"][:, 1]
-        R.load_contact_impulses(sr.world, imp)
-        if len(oj):
-            jimp = np.zeros((len(oj), 5), dtype=np.float32)
-            jimp[:, 0:2] = oj["impulse"]
-            jimp[:, 2] = oj["motorImpulse"]
-            jimp[:, 3] = oj["lowerImpulse"]
-            jimp[:, 4] = oj["upperImpulse"]
-            R.load_joint_impulses(sr.world, jimp)
-        R.step_finalize(sr.world)
-
-        # compare
-        post = dw.download_all_bodies(cap)
-        rf, ri = R.bodies(sr.world)
-        v = ri[:, 0] == 1
-        for name, col, width in (("position", F["position"], 2), ("rot", F["rot"], 2), ("linearVelocity", F["v"], 2),
-                                 ("origin", F["origin"], 2)):
-            g = np.ascontiguousarray(post[name][v]).reshape(int(v.sum()), -1)
-            o = np.ascontiguousarray(rf[v, col:col + width])
-            if not bit_equal(g, o):
-                worst[name] = max(worst.get(name, 0.0), float(np.abs(g - o).max()))
-        if not bit_equal(post["angularVelocity"][v], rf[v, F["w"]]):
-            worst["w"] = max(worst.get("w", 0.0), float(np.abs(post["angularVelocity"][v] - rf[v, F["w"]]).max()))
-        live = rows_key["pointCount"] > 0
-        for name in ("normalImpulse", "tangentImpulse"):
-            if not bit_equal(got_contacts["points"][name][live], oc["points"][name][live]):
-                worst[name] = max(worst.get(name, 0.0), float(np.abs(got_contacts["points"][name][live] - oc["points"][name][live]).max()))
-        if len(oj):
-            got_joints = dw.download_joints(len(oj))
-            jlive = (joints["flags"] & 1) == 1
-            for name in ("impulse", "motorImpulse", "lowerImpulse", "upperImpulse"):
-                if not bit_equal(got_joints[name][jlive], oj[name][jlive]):
-                    worst["joint " + name] = 1.0
-        assert not worst, f"{solver} step {step}: device != reference pipeline replayed in the device's order: {worst}"
+        got = np.frombuffer(device_step_digest(dw), dtype=np.uint8)
+        assert np.array_equal(got, want[step]), \
+            f"{solver} step {step}: device != reference pipeline replayed in the device's order"
     c = dw.counters()
     assert c.graphReplays >= min_replays, f"the solver stage was replayed as a graph only {c.graphReplays} times"
-    sr.destroy()
     sp.destroy()
     return c
 
 
-def test_config1_every_step_bit_exact(reference, product, dev):
+def _falling_boxes(lib, solver, **kw):
+    sc = scenes.vertical_stack(lib, solver, count=5, columns=4)
+    for k, bid in enumerate(sc.bodies[1:]):
+        if k % 5 >= 3:
+            lib.s2Body_SetLinearVelocity(bid, capi.Vec2(3.0 if (k // 5) % 2 == 0 else -3.0, 1.0))
+    return sc
+
+
+def _kinematic_platforms(lib, solver, **kw):
+    import ctypes as C
+    world = lib.create_world(solver)
+    sc = scenes.Scene(lib, world, name="kinematic_platforms")
+    h, base = 0.5, 16
+    box = lib.s2MakeSquare(h)
+    sd = scenes.default_shape_def()
+    sd.density = 1.0
+    for k in range(4):
+        x0 = k * 30.0
+        bd = scenes.default_body_def()
+        bd.type = capi.KINEMATIC_BODY
+        bd.position = capi.Vec2(x0, -1.0)
+        bd.linearVelocity = capi.Vec2(0.6 if k % 2 == 0 else -0.4, 0.0)
+        gid = lib.s2CreateBody(world, C.byref(bd))
+        plat = lib.s2MakeBox(0.5 * base + 2.0, 1.0)
+        lib.s2CreatePolygonShape(gid, C.byref(sd), C.byref(plat))
+        sc.bodies.append(gid)
+        bd = scenes.default_body_def()
+        bd.type = capi.DYNAMIC_BODY
+        for i in range(base):
+            y = (2.0 * i + 1.0) * h
+            for j in range(i, base):
+                x = (i + 1.0) * h + 2.0 * (j - i) * h - h * base
+                bd.position = capi.Vec2(x0 + x, y)
+                bid = lib.s2CreateBody(world, C.byref(bd))
+                lib.s2CreatePolygonShape(bid, C.byref(sd), C.byref(box))
+                sc.bodies.append(bid)
+    return sc
+
+
+def _force_regions(dw):
+    dw.set_regions(2)
+
+
+VARIANTS = ["PGS", "PGS_NGS", "PGS_NGS_Block", "PGS_Soft", "SoftStep", "TGS_NGS", "XPBD"]
+# name -> (recipe, solver, steps, velocity iterations, relax iterations, recipe kwargs, device setup)
+CASES = {
+    "config1": (scenes.pyramid, "TGS_Soft", 120, 4, 2, dict(base_count=10), None),
+    "pyramid_5k": (scenes.pyramid, "TGS_Soft", 60, 4, 2, dict(base_count=100), None),
+    "joints_and_contacts": (scenes.joint_contact_stress, "TGS_Soft", 90, 4, 2, dict(bridges=3, planks=24, grid=9), None),
+    "falling_boxes": (_falling_boxes, "TGS_Soft", 120, 4, 2, {}, None),
+    "kinematic_platforms": (_kinematic_platforms, "TGS_Soft", 40, 4, 2, {}, _force_regions),
+}
+CASES.update({f"variant_{s.lower()}": (scenes.pyramid, s, 40, 4, 2, dict(base_count=20), None) for s in VARIANTS})
+
+
+def test_config1_every_step_bit_exact(product, dev):
     """BASELINE config 1 (Pyramid, 55 boxes, TGS_Soft, 4 sub-steps), 120 free-running steps."""
-    c = _run(reference, product, dev, scenes.pyramid, "TGS_Soft", 120, 4, 2, dict(base_count=10), min_replays=60)
+    c = _run(product, dev, "config1", min_replays=60)
     assert c.constraintCount > 100
 
 
-def test_pyramid_5k_every_step_bit_exact(reference, product, dev):
+def test_pyramid_5k_every_step_bit_exact(product, dev):
     """5 050 boxes / ~15 000 contact constraints, 60 free-running steps: several thread blocks, contact-table changes while
     the pile settles, graph replays with the schedule skipped in between."""
-    c = _run(reference, product, dev, scenes.pyramid, "TGS_Soft", 60, 4, 2, dict(base_count=100))
+    c = _run(product, dev, "pyramid_5k")
     assert c.constraintCount > 14000
 
 
-def test_joints_and_contacts_every_step_bit_exact(reference, product, dev):
+def test_joints_and_contacts_every_step_bit_exact(product, dev):
     """Bridges (revolute chains) with boxes dropped on them: joints and contacts in one colouring, contacts appearing and
     disappearing every few steps."""
-    c = _run(reference, product, dev, scenes.joint_contact_stress, "TGS_Soft", 90, 4, 2, dict(bridges=3, planks=24, grid=9))
+    c = _run(product, dev, "joints_and_contacts")
     assert c.jointCount == 75
 
 
-@pytest.mark.parametrize("solver", ["PGS", "PGS_NGS", "PGS_NGS_Block", "PGS_Soft", "SoftStep", "TGS_NGS", "XPBD"])
-def test_variants_every_step_bit_exact(reference, product, dev, solver):
-    c = _run(reference, product, dev, scenes.pyramid, solver, 40, 4, 2, dict(base_count=20))
+@pytest.mark.parametrize("solver", VARIANTS)
+def test_variants_every_step_bit_exact(product, dev, solver):
+    c = _run(product, dev, f"variant_{solver.lower()}")
     assert c.constraintCount > 300
 
 
-def test_falling_boxes_every_step_bit_exact(reference, product, dev):
+def test_falling_boxes_every_step_bit_exact(product, dev):
     """Boxes thrown sideways: proxies leave their fat AABBs, pairs are created and destroyed, manifolds gain and lose
     points — the schedule is rebuilt on exactly the steps the device flags."""
-    def recipe(lib, solver, **kw):
-        sc = scenes.vertical_stack(lib, solver, count=5, columns=4)
-        for k, bid in enumerate(sc.bodies[1:]):
-            if k % 5 >= 3:
-                lib.s2Body_SetLinearVelocity(bid, capi.Vec2(3.0 if (k // 5) % 2 == 0 else -3.0, 1.0))
-        return sc
-    c = _run(reference, product, dev, recipe, "TGS_Soft", 120, 4, 2, {})
+    c = _run(product, dev, "falling_boxes")
     assert c.pairPassCount > 5
 
 
-def test_kinematic_platforms_under_regions_every_step_bit_exact(reference, product, dev):
+def test_kinematic_platforms_under_regions_every_step_bit_exact(product, dev):
     """Piles standing on KINEMATIC platforms that slide sideways, region-local schedule forced. A kinematic body conflicts
     with nothing (no constraint moves it) but its pose changes every sub-step, integrated by the block that owns it: a
     constraint that reads it from another block's region-local phase would race with that pass. Such constraints have to
     run in the device-wide steps (s2bClassifyItemsKernel)."""
-    def recipe(lib, solver, **kw):
-        import ctypes as C
-        world = lib.create_world(solver)
-        sc = scenes.Scene(lib, world, name="kinematic_platforms")
-        h, base = 0.5, 16
-        box = lib.s2MakeSquare(h)
-        sd = scenes.default_shape_def()
-        sd.density = 1.0
-        for k in range(4):
-            x0 = k * 30.0
-            bd = scenes.default_body_def()
-            bd.type = capi.KINEMATIC_BODY
-            bd.position = capi.Vec2(x0, -1.0)
-            bd.linearVelocity = capi.Vec2(0.6 if k % 2 == 0 else -0.4, 0.0)
-            gid = lib.s2CreateBody(world, C.byref(bd))
-            plat = lib.s2MakeBox(0.5 * base + 2.0, 1.0)
-            lib.s2CreatePolygonShape(gid, C.byref(sd), C.byref(plat))
-            sc.bodies.append(gid)
-            bd = scenes.default_body_def()
-            bd.type = capi.DYNAMIC_BODY
-            for i in range(base):
-                y = (2.0 * i + 1.0) * h
-                for j in range(i, base):
-                    x = (i + 1.0) * h + 2.0 * (j - i) * h - h * base
-                    bd.position = capi.Vec2(x0 + x, y)
-                    bid = lib.s2CreateBody(world, C.byref(bd))
-                    lib.s2CreatePolygonShape(bid, C.byref(sd), C.byref(box))
-                    sc.bodies.append(bid)
-        return sc
-    c = _run(reference, product, dev, recipe, "TGS_Soft", 40, 4, 2, {}, setup=lambda dw: dw.set_regions(2))
+    c = _run(product, dev, "kinematic_platforms")
     assert c.regionCount >= 3 and c.cutCount >= 40

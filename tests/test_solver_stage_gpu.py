@@ -1,8 +1,8 @@
 """GPU parity of the solver stage (s2Solve_* on the device) against the unmodified reference.
 
-Each case: build a scene in the reference, run some steps, then take ONE step split at the stage boundaries:
-collide on the reference -> mirror bodies + manifolds (pool order) into a device world -> solver stage on both ->
-compare per-body state and stored impulses.
+Each case: a scene stepped by the reference, then ONE step split at the stage boundaries, recorded in tests/golden/stage:
+the bodies + manifolds (pool order) the reference's solver stage received -> a device world -> solver stage ->
+compare per-body state and stored impulses with what the reference's solver stage returned.
 
 * WAVEFRONT schedule preserves the reference's sequential Gauss-Seidel order; the kernels are compiled with
   -fmad=false, so the result must be BIT-EXACT (tolerance 0).
@@ -13,67 +13,61 @@ compare per-body state and stored impulses.
 import numpy as np
 import pytest
 
-from helpers import bit_equal, compare_bodies, load_device_world_from_ref
-from oracle import ref as refmod
-from solver2d_b200 import capi, device, scenes
+from helpers import bit_equal
+from solver2d_b200 import capi, device
+from stage_cases import load_case
 
 pytestmark = pytest.mark.gpu
 
 DT = 1.0 / 60.0
 
 
-def _one_case(reference, dev, recipe, solver, warm_steps, vel_iters, pos_iters, schedule, persistent, warm_start=True, **kw):
-    R = reference
-    sc = recipe(R, solver, **kw)
-    for _ in range(warm_steps):
-        sc.step(DT, vel_iters, pos_iters, True)
-    R.step_collide(sc.world)
-    dw = load_device_world_from_ref(dev, R, sc.world, solver)
+def _one_case(dev, recipe, solver, warm_steps, vel_iters, pos_iters, schedule, persistent, warm_start=True, warm_iters=None,
+              **kw):
+    """The rows the reference's solver stage received (tests/golden/stage) -> a device world -> solver stage -> compare
+    per-body state and stored impulses with what the reference's stage returned."""
+    case = load_case(recipe, solver, warm_steps, vel_iters, pos_iters, warm_start, warm_iters, **kw)
+    dw = dev.create_world(capi.SOLVER[solver])
+    dw.upload_bodies(case.bodies, len(case.bodies))
+    dw.upload_joints(case.joints, len(case.joints))
+    dw.upload_contacts(case.contacts)
     dw.set_schedule(schedule)
-    dw.set_persistent(persistent)
+    if persistent is not None:
+        dw.set_persistent(persistent)
     ctx = device.make_context(solver, DT, vel_iters, pos_iters, warm_start)
 
-    R.step_solve(sc.world, DT, vel_iters, pos_iters, warm_start)
-    bf, bi = R.bodies(sc.world)
-    cf, ci = R.contacts(sc.world)
-
     dw.solve(ctx)
-    rows = dw.download_all_bodies(bf.shape[0])
-    contacts = dw.download_contacts(len(dw.ref_contact_slots))
+    rows = dw.download_all_bodies(len(case.bodies))
+    contacts = dw.download_contacts(len(case.contacts))
     counters = dw.counters()
-    diff = compare_bodies(rows, bf, bi)
+    valid = (case.bodies["flags"] & 1) == 1
+    diff = {key: float(np.abs(rows[name][valid] - case.out(name)[valid]).max()) if valid.any() else 0.0
+            for key, name in (("pos", "position"), ("rot", "rot"), ("v", "linearVelocity"), ("w", "angularVelocity"),
+                              ("origin", "origin"))}
 
     # stored impulses, same (pool) order on both sides
-    P = refmod.POINT_F
-    ref_imp = np.stack([cf[dw.ref_contact_slots, refmod.CONTACT_F["points"] + refmod.POINT_STRIDE * j + P["normalImpulse"]]
-                        for j in range(2)], axis=1)
+    ref_imp, ref_timp = case.out_normal, case.out_tangent
     dev_imp = contacts["points"]["normalImpulse"]
-    ref_timp = np.stack([cf[dw.ref_contact_slots, refmod.CONTACT_F["points"] + refmod.POINT_STRIDE * j + P["tangentImpulse"]]
-                         for j in range(2)], axis=1)
     dev_timp = contacts["points"]["tangentImpulse"]
     two = np.stack([contacts["pointCount"] > 0, contacts["pointCount"] > 1], axis=1) if len(contacts) else None
     diff["impulse"] = float(np.abs(ref_imp - dev_imp).max()) if len(contacts) else 0.0
-    valid = bi[:, 0] == 1
-    F = refmod.BODY_F
-    exact = (bit_equal(rows["position"][valid], bf[valid, F["position"]:F["position"] + 2])
-             and bit_equal(rows["linearVelocity"][valid], bf[valid, F["v"]:F["v"] + 2])
-             and bit_equal(rows["angularVelocity"][valid], bf[valid, F["w"]])
-             and bit_equal(rows["rot"][valid], bf[valid, F["rot"]:F["rot"] + 2])
+    exact = (bit_equal(rows["position"][valid], case.out("position")[valid])
+             and bit_equal(rows["linearVelocity"][valid], case.out("linearVelocity")[valid])
+             and bit_equal(rows["angularVelocity"][valid], case.out("angularVelocity")[valid])
+             and bit_equal(rows["rot"][valid], case.out("rot")[valid])
              and bit_equal(ref_imp, dev_imp)
              and (two is None or bit_equal(ref_timp[two], dev_timp[two])))
     if solver == "TGS_Sticky" and len(contacts):
         live = contacts["pointCount"] > 0
-        exact = exact and bool(np.array_equal(contacts["frictionPersisted"][live],
-                                              ci[dw.ref_contact_slots, refmod.CONTACT_I["frictionPersisted"]][live]))
+        exact = exact and bool(np.array_equal(contacts["frictionPersisted"][live], case.out_friction_persisted[live]))
     dw.destroy()
-    sc.destroy()
     return diff, exact, counters
 
 
 @pytest.mark.parametrize("persistent", [True, False])
 @pytest.mark.parametrize("base,warm", [(10, 0), (10, 30), (40, 5)])
-def test_tgs_soft_wavefront_bit_exact(reference, dev, base, warm, persistent):
-    diff, exact, counters = _one_case(reference, dev, scenes.pyramid, "TGS_Soft", warm, 4, 2, device.SCHEDULE_WAVEFRONT,
+def test_tgs_soft_wavefront_bit_exact(dev, base, warm, persistent):
+    diff, exact, counters = _one_case(dev, "pyramid", "TGS_Soft", warm, 4, 2, device.SCHEDULE_WAVEFRONT,
                                       persistent, base_count=base)
     assert counters.constraintCount > 0
     assert exact, f"not bit-exact: {diff}"
@@ -81,8 +75,8 @@ def test_tgs_soft_wavefront_bit_exact(reference, dev, base, warm, persistent):
 
 
 @pytest.mark.parametrize("persistent", [True, False])
-def test_tgs_soft_color_close(reference, dev, persistent):
-    diff, exact, counters = _one_case(reference, dev, scenes.pyramid, "TGS_Soft", 30, 4, 2, device.SCHEDULE_COLOR,
+def test_tgs_soft_color_close(dev, persistent):
+    diff, exact, counters = _one_case(dev, "pyramid", "TGS_Soft", 30, 4, 2, device.SCHEDULE_COLOR,
                                       persistent, base_count=20)
     assert 1 <= counters.groupCount <= 16
     assert counters.overflowCount == 0
@@ -90,22 +84,10 @@ def test_tgs_soft_color_close(reference, dev, persistent):
     assert diff["pos"] < 2e-3 and diff["v"] < 0.2, diff
 
 
-def test_tgs_soft_no_warm_start_and_no_relax(reference, dev):
-    R = reference
-    sc = scenes.pyramid(R, "TGS_Soft", base_count=12)
-    for _ in range(10):
-        sc.step(DT, 4, 2, True)
-    R.step_collide(sc.world)
-    dw = load_device_world_from_ref(dev, R, sc.world, "TGS_Soft")
-    dw.set_schedule(device.SCHEDULE_WAVEFRONT)
-    ctx = device.make_context("TGS_Soft", DT, 3, 0, False)
-    R.step_solve(sc.world, DT, 3, 0, False)
-    bf, bi = R.bodies(sc.world)
-    dw.solve(ctx)
-    rows = dw.download_all_bodies(bf.shape[0])
-    assert max(compare_bodies(rows, bf, bi).values()) == 0.0
-    dw.destroy()
-    sc.destroy()
+def test_tgs_soft_no_warm_start_and_no_relax(dev):
+    diff, exact, counters = _one_case(dev, "pyramid", "TGS_Soft", 10, 3, 0, device.SCHEDULE_WAVEFRONT, None,
+                                      warm_start=False, warm_iters=(4, 2), base_count=12)
+    assert max(v for k, v in diff.items() if k != "impulse") == 0.0
 
 
 VARIANTS = ["Jacobi", "PGS", "PGS_NGS", "PGS_NGS_Block", "PGS_Soft", "SoftStep", "TGS_Sticky", "TGS_Soft", "TGS_NGS", "XPBD"]
@@ -113,24 +95,24 @@ VARIANTS = ["Jacobi", "PGS", "PGS_NGS", "PGS_NGS_Block", "PGS_Soft", "SoftStep",
 
 @pytest.mark.parametrize("persistent", [True, False])
 @pytest.mark.parametrize("solver", VARIANTS)
-def test_variant_wavefront_bit_exact_pyramid(reference, dev, solver, persistent):
+def test_variant_wavefront_bit_exact_pyramid(dev, solver, persistent):
     warm = 2 if solver == "Jacobi" else 30  # the reference's Jacobi blows a pyramid apart within five steps
-    diff, exact, counters = _one_case(reference, dev, scenes.pyramid, solver, warm, 4, 2, device.SCHEDULE_WAVEFRONT,
+    diff, exact, counters = _one_case(dev, "pyramid", solver, warm, 4, 2, device.SCHEDULE_WAVEFRONT,
                                       persistent, base_count=12)
     assert counters.constraintCount > 50
     assert exact, f"{solver} not bit-exact: {diff}"
 
 
 @pytest.mark.parametrize("solver", VARIANTS)
-def test_variant_wavefront_bit_exact_joints(reference, dev, solver):
-    diff, exact, counters = _one_case(reference, dev, scenes.limited_chains, solver, 40, 4, 2, device.SCHEDULE_WAVEFRONT, True)
+def test_variant_wavefront_bit_exact_joints(dev, solver):
+    diff, exact, counters = _one_case(dev, "limited_chains", solver, 40, 4, 2, device.SCHEDULE_WAVEFRONT, True)
     assert counters.jointCount == 19
     assert exact, f"{solver} not bit-exact: {diff}"
 
 
 @pytest.mark.parametrize("solver", VARIANTS)
-def test_variant_wavefront_bit_exact_cold_mixed(reference, dev, solver):
-    diff, exact, counters = _one_case(reference, dev, scenes.mixed_shapes, solver, 100, 3, 1, device.SCHEDULE_WAVEFRONT, True,
+def test_variant_wavefront_bit_exact_cold_mixed(dev, solver):
+    diff, exact, counters = _one_case(dev, "mixed_shapes", solver, 100, 3, 1, device.SCHEDULE_WAVEFRONT, True,
                                       warm_start=False)
     assert counters.constraintCount > 20
     assert exact, f"{solver} not bit-exact: {diff}"
