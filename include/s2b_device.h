@@ -170,7 +170,7 @@ typedef struct s2bCounters
 	int32_t jointCount;		 // live joints in the last solve
 	int32_t groupCount;		 // colours (or wavefront levels) in the last solve
 	int32_t overflowCount;	 // constraints solved serially after the coloured groups
-	int32_t treeHeight;		 // depth of the last BVH
+	int32_t treeHeight;		 // box levels a pair query descends through, leaves included (broad-phase hierarchy of the last pass)
 	int32_t movedCount;		 // proxies whose fat AABB changed in the last finalize
 	int32_t pairPassCount;	 // number of broad-phase passes run so far
 	int32_t kernelLaunches;	 // CUDA kernels launched by this world since creation (graph replays count their kernels)
@@ -181,6 +181,8 @@ typedef struct s2bCounters
 	int32_t cutCount;		 // constraints that straddle two regions (solved in device-wide steps)
 	int32_t cutGroupCount;	 // colours of the cut set = device-wide steps per Gauss-Seidel sweep
 	int32_t recolouredCount; /* constraints moved out of a sparse top colour by Kempe chains so far (colouring, DESIGN.md 3.2) */
+	int32_t largeLeafCount;	 // scene-sized proxies kept out of the broad-phase hierarchy (DESIGN.md 3.3)
+	int32_t pairRebuildCount; // broad-phase passes that re-sorted the proxies so far
 } s2bCounters;
 
 // ---- lifecycle ------------------------------------------------------------------------------------------------

@@ -5,9 +5,11 @@
 // hash set (src/table.c) and the fat-AABB overlap test + s2DestroyContact of world.c:149-166.
 //
 // B200-first design instead of a port of the pointer-chasing tree:
-//   * a linear BVH (Morton order + Karras radix tree) over ALL proxies is rebuilt from scratch, fully in parallel,
-//     only on steps where some proxy left its fat AABB (or the host created/destroyed something);
-//   * one thread per *moved* proxy walks the BVH and applies the reference's pair rules (both-moved de-duplication by
+//   * the proxies are sorted in Morton order, fully in parallel, only on steps where some proxy left its fat AABB (or the
+//     host created/destroyed something); a shallow 16-wide hierarchy over that order (node i of level l covers sorted
+//     leaves [i*16^l, (i+1)*16^l)) is refitted every pass, and the few scene-sized proxies are kept out of it in a short
+//     list that every query tests directly;
+//   * one thread per *moved* proxy walks the hierarchy and applies the reference's pair rules (both-moved de-duplication by
 //     proxy key, body-type rules of the three-tree query, existing pair, same body, filter, joint override, shape-type
 //     table) — so the set of created contacts equals the reference's;
 //   * existing contacts whose fat AABBs stopped overlapping are dropped, survivors and new pairs are merged by a radix
@@ -26,15 +28,11 @@ struct BroadScratch
 	DevArray<int> leafShape;	   // compacted valid shapes
 	DevArray<unsigned> mortonIn, mortonOut;
 	DevArray<int> leafIn, leafOut; // sorted leaf -> index into leafShape
-	DevArray<int> counters;		   // [0] leaf count [1] new pair count [2] kept count [3] bounds ready ...
-	DevArray<int> boundsBits;	   // 4 ordered-int encoded floats: min.x min.y max.x max.y
-	DevArray<int2> children;	   // internal nodes
-	DevArray<int> parent;		   // all nodes (internal [0,n-1), leaves [n-1, 2n-1))
-	DevArray<float4> nodeBox;	   // all nodes
-	DevArray<float4> pairBox;	   // per internal node: the boxes of its two children, adjacent
-	DevArray<int> visit;		   // refit arrival counters (internal nodes)
-	DevArray<int> nodeHeight;
-	DevArray<int> movedLeaves;	   // sorted-leaf indices of moved proxies
+	DevArray<int> sortedShape;	   // sorted leaf -> shape slot (leafShape[leafOut[k]], composed at the rebuild)
+	DevArray<int> counters;		   // BC_*
+	DevArray<int> boundsBits;	   // 8 ordered-int encoded floats: box centres min.x min.y max.x max.y, boxes min.x min.y max.x max.y
+	DevArray<float4> nodeBox;	   // sorted leaf boxes [0, n), then the levels of the hierarchy (s2bLevels)
+	DevArray<int> movedShapes;	   // shapes of the moved proxies, in Morton order
 	DevArray<int> movedFlag;
 	DevArray<int> largeShapes;	   // shapes of moved proxies with scene-sized boxes
 	DevArray<unsigned long long> newKey;
@@ -88,14 +86,11 @@ void s2bFreeBroadScratch(s2bWorld* w)
 	b->mortonOut.release();
 	b->leafIn.release();
 	b->leafOut.release();
+	b->sortedShape.release();
 	b->counters.release();
 	b->boundsBits.release();
-	b->children.release();
-	b->parent.release();
 	b->nodeBox.release();
-	b->visit.release();
-	b->nodeHeight.release();
-	b->movedLeaves.release();
+	b->movedShapes.release();
 	b->movedFlag.release();
 	b->newKey.release();
 	b->newShapes.release();
@@ -106,7 +101,6 @@ void s2bFreeBroadScratch(s2bWorld* w)
 	b->mergeSrcIn.release();
 	b->mergeSrcOut.release();
 	b->cubTemp.release();
-	b->pairBox.release();
 	b->largeShapes.release();
 	b->pairHash.release();
 	for (int i = 0; i < 2; ++i)
@@ -124,14 +118,18 @@ void s2bFreeBroadScratch(s2bWorld* w)
 	w->broad = nullptr;
 }
 
+// BC_LEAVES and BC_LARGE_LEAVES describe the sorted order and live as long as it is reused; the others are cleared by
+// every pass
 enum
 {
 	BC_LEAVES = 0,
-	BC_NEW_PAIRS = 1,
-	BC_KEPT = 2,
-	BC_MOVED = 3,
-	BC_HEIGHT = 4,
-	BC_LARGE = 5, // moved proxies handled by the leaf-side query
+	BC_LARGE_LEAVES = 1, // scene-sized leaves kept out of the hierarchy at the last rebuild (may exceed the list's capacity)
+	BC_NEW_PAIRS = 2,
+	BC_KEPT = 3,
+	BC_MOVED = 4,
+	BC_HEIGHT = 5,
+	BC_LARGE = 6,		// moved proxies handled by the leaf-side query
+	BC_REFIT_DONE = 7,	// blocks of s2bRefit that finished their part
 	BC_SIZE = 8
 };
 
@@ -299,8 +297,62 @@ __device__ __forceinline__ int s2bPairKind(int t1, int t2)
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// BVH build
+// hierarchy
 // ---------------------------------------------------------------------------------------------------------------
+
+// A fixed-fanout hierarchy over the Morton-sorted leaves: node i of level l covers sorted leaves [i*16^l, (i+1)*16^l), so
+// the topology is implicit in the order and a rebuild is the sort alone. At 100 k leaves a query descends 5 levels of
+// independent 16-box tests instead of the dozens of dependent levels of a binary radix tree.
+#define S2B_FANOUT 16
+#define S2B_MAX_LEVELS 8 // 16^8 leaves
+
+// Leaves whose fat box is scene-sized (the pyramid's ground is 547 m wide) would make every ancestor scene-sized and drag
+// every query down their chain. At a rebuild up to S2B_MAX_LARGE_LEAVES of them sort behind the hierarchy's leaves
+// (sorted leaves [n - large, n)); every query tests them directly. Any beyond the capacity stay in the hierarchy. Each leaf
+// is on exactly one side, so every (query, leaf) overlap is still considered exactly once.
+#define S2B_MAX_LARGE_LEAVES 64
+
+// Offsets into nodeBox and node counts of the levels over the first nh sorted leaves: level 0 (the leaves) at 0, level 1 at
+// n, each next level right behind the previous one. Returns the top level: the first whose node count is <= 16 (0 when
+// the leaves themselves are that few). s2bRefit and s2bFindPairs both lay the levels out with this.
+__device__ __forceinline__ int s2bLevels(int n, int nh, int* offset, int* count)
+{
+	offset[0] = 0;
+	count[0] = nh;
+	int top = 0, off = n;
+	while (count[top] > S2B_FANOUT && top + 1 < S2B_MAX_LEVELS)
+	{
+		int c = (count[top] + S2B_FANOUT - 1) / S2B_FANOUT;
+		top += 1;
+		offset[top] = off;
+		count[top] = c;
+		off += c;
+	}
+	return top;
+}
+
+__device__ __forceinline__ float4 s2bEmptyBox()
+{
+	return make_float4(3.0e38f, 3.0e38f, -3.0e38f, -3.0e38f);
+}
+
+__device__ __forceinline__ float4 s2bUnion(float4 a, float4 b)
+{
+	return make_float4(fminf(a.x, b.x), fminf(a.y, b.y), fmaxf(a.z, b.z), fmaxf(a.w, b.w));
+}
+
+// union over the 16 lanes of each half warp (every lane of the warp has to call this)
+__device__ __forceinline__ float4 s2bUnion16(float4 box)
+{
+	for (int o = S2B_FANOUT / 2; o > 0; o >>= 1)
+	{
+		box.x = fminf(box.x, __shfl_xor_sync(0xFFFFFFFFu, box.x, o));
+		box.y = fminf(box.y, __shfl_xor_sync(0xFFFFFFFFu, box.y, o));
+		box.z = fmaxf(box.z, __shfl_xor_sync(0xFFFFFFFFu, box.z, o));
+		box.w = fmaxf(box.w, __shfl_xor_sync(0xFFFFFFFFu, box.w, o));
+	}
+	return box;
+}
 
 __global__ void s2bFlagValidShapes(ShapeView s, int* validFlag)
 {
@@ -311,35 +363,46 @@ __global__ void s2bFlagValidShapes(ShapeView s, int* validFlag)
 	}
 }
 
+// bounds of the box centres (Morton quantisation) and of the boxes themselves (what counts as scene-sized)
 __global__ void s2bSceneBounds(ShapeView s, const int* leafShape, const int* counters, int* boundsBits)
 {
 	int n = counters[BC_LEAVES];
 	int k = blockIdx.x * blockDim.x + threadIdx.x;
-	float minx = 3.0e38f, miny = 3.0e38f, maxx = -3.0e38f, maxy = -3.0e38f;
+	float c[4] = {3.0e38f, 3.0e38f, -3.0e38f, -3.0e38f};
+	float4 box = s2bEmptyBox();
 	if (k < n)
 	{
-		float4 f = s.fat[leafShape[k]];
-		float cx = 0.5f * (f.x + f.z), cy = 0.5f * (f.y + f.w);
-		minx = maxx = cx;
-		miny = maxy = cy;
+		box = s.fat[leafShape[k]];
+		float cx = 0.5f * (box.x + box.z), cy = 0.5f * (box.y + box.w);
+		c[0] = c[2] = cx;
+		c[1] = c[3] = cy;
 	}
+	float v[8] = {c[0], c[1], c[2], c[3], box.x, box.y, box.z, box.w};
 	for (int o = 16; o > 0; o >>= 1)
 	{
-		minx = fminf(minx, __shfl_xor_sync(0xFFFFFFFFu, minx, o));
-		miny = fminf(miny, __shfl_xor_sync(0xFFFFFFFFu, miny, o));
-		maxx = fmaxf(maxx, __shfl_xor_sync(0xFFFFFFFFu, maxx, o));
-		maxy = fmaxf(maxy, __shfl_xor_sync(0xFFFFFFFFu, maxy, o));
+		for (int j = 0; j < 8; ++j)
+		{
+			float u = __shfl_xor_sync(0xFFFFFFFFu, v[j], o);
+			v[j] = (j & 2) ? fmaxf(v[j], u) : fminf(v[j], u);
+		}
 	}
 	if ((threadIdx.x & 31) == 0)
 	{
-		atomicMin(boundsBits + 0, s2bFloatToOrdered(minx));
-		atomicMin(boundsBits + 1, s2bFloatToOrdered(miny));
-		atomicMax(boundsBits + 2, s2bFloatToOrdered(maxx));
-		atomicMax(boundsBits + 3, s2bFloatToOrdered(maxy));
+		for (int j = 0; j < 8; ++j)
+		{
+			if (j & 2)
+			{
+				atomicMax(boundsBits + j, s2bFloatToOrdered(v[j]));
+			}
+			else
+			{
+				atomicMin(boundsBits + j, s2bFloatToOrdered(v[j]));
+			}
+		}
 	}
 }
 
-__global__ void s2bMortonCodes(ShapeView s, const int* leafShape, const int* counters, const int* boundsBits, unsigned* morton,
+__global__ void s2bMortonCodes(ShapeView s, const int* leafShape, int* counters, const int* boundsBits, unsigned* morton,
 							   int* leafIndex, int capacity)
 {
 	int n = counters[BC_LEAVES];
@@ -348,128 +411,40 @@ __global__ void s2bMortonCodes(ShapeView s, const int* leafShape, const int* cou
 	{
 		return;
 	}
+	leafIndex[k] = k;
 	if (k >= n)
 	{
-		morton[k] = 0xFFFFFFFFu; // padding sorts last
-		leafIndex[k] = k;
+		morton[k] = 0xFFFFFFFFu; // padding sorts last (behind the large leaves: the sort is stable)
 		return;
 	}
 	float minx = s2bOrderedToFloat(boundsBits[0]), miny = s2bOrderedToFloat(boundsBits[1]);
 	float maxx = s2bOrderedToFloat(boundsBits[2]), maxy = s2bOrderedToFloat(boundsBits[3]);
 	float4 f = s.fat[leafShape[k]];
+	if (n >= 256)
+	{
+		float sceneSide = fmaxf(s2bOrderedToFloat(boundsBits[6]) - s2bOrderedToFloat(boundsBits[4]),
+								s2bOrderedToFloat(boundsBits[7]) - s2bOrderedToFloat(boundsBits[5]));
+		float side = fmaxf(f.z - f.x, f.w - f.y);
+		if (side * 16.0f > sceneSide && atomicAdd(counters + BC_LARGE_LEAVES, 1) < S2B_MAX_LARGE_LEAVES)
+		{
+			morton[k] = 0xFFFFFFFFu; // ordinary codes are below 2^31
+			return;
+		}
+	}
 	float cx = 0.5f * (f.x + f.z), cy = 0.5f * (f.y + f.w);
 	float ex = fmaxf(maxx - minx, 1.0e-6f), ey = fmaxf(maxy - miny, 1.0e-6f);
 	float ux = fminf(fmaxf((cx - minx) / ex, 0.0f), 1.0f);
 	float uy = fminf(fmaxf((cy - miny) / ey, 0.0f), 1.0f);
 	unsigned qx = (unsigned)(ux * 32767.0f), qy = (unsigned)(uy * 32767.0f);
 	morton[k] = (s2bExpandBits(qx) | (s2bExpandBits(qy) << 1)) & 0x7FFFFFFFu;
-	leafIndex[k] = k;
 }
 
-// common-prefix length of sorted keys i and j; ties on the code are broken by the position (Karras 2012)
-__device__ __forceinline__ int s2bDelta(const unsigned* codes, int n, int i, int j)
+__global__ void s2bSortedShapes(const int* leafShape, const int* leafOut, const int* counters, int* sortedShape)
 {
-	if (j < 0 || j >= n)
-	{
-		return -1;
-	}
-	unsigned a = codes[i], b = codes[j];
-	if (a == b)
-	{
-		return 32 + __clz((unsigned)i ^ (unsigned)j);
-	}
-	return __clz(a ^ b);
-}
-
-__global__ void s2bBuildRadixTree(const unsigned* codes, const int* counters, int2* children, int* parent)
-{
-	int n = counters[BC_LEAVES];
-	int i = blockIdx.x * blockDim.x + threadIdx.x;
-	if (i >= n - 1)
-	{
-		return;
-	}
-	int d = (s2bDelta(codes, n, i, i + 1) - s2bDelta(codes, n, i, i - 1)) >= 0 ? 1 : -1;
-	int deltaMin = s2bDelta(codes, n, i, i - d);
-	int lmax = 2;
-	while (s2bDelta(codes, n, i, i + lmax * d) > deltaMin)
-	{
-		lmax <<= 1;
-	}
-	int l = 0;
-	for (int t = lmax >> 1; t >= 1; t >>= 1)
-	{
-		if (s2bDelta(codes, n, i, i + (l + t) * d) > deltaMin)
-		{
-			l += t;
-		}
-	}
-	int j = i + l * d;
-	int deltaNode = s2bDelta(codes, n, i, j);
-	int s = 0;
-	int t = l;
-	do
-	{
-		t = (t + 1) >> 1;
-		if (s2bDelta(codes, n, i, i + (s + t) * d) > deltaNode)
-		{
-			s += t;
-		}
-	} while (t > 1);
-	int gamma = i + s * d + min(d, 0);
-	int left = min(i, j) == gamma ? (n - 1) + gamma : gamma;
-	int right = max(i, j) == gamma + 1 ? (n - 1) + gamma + 1 : gamma + 1;
-	children[i] = make_int2(left, right);
-	parent[left] = i;
-	parent[right] = i;
-	if (i == 0)
-	{
-		parent[0] = -1;
-	}
-}
-
-__global__ void s2bRefit(ShapeView s, const int* leafShape, const int* sortedLeaf, const int* counters, const int2* children,
-						 const int* parent, float4* nodeBox, float4* pairBox, int* visit, int* nodeHeight, int* countersOut)
-{
-	int n = counters[BC_LEAVES];
 	int k = blockIdx.x * blockDim.x + threadIdx.x;
-	if (k >= n)
+	if (k < counters[BC_LEAVES])
 	{
-		return;
-	}
-	int node = (n - 1) + k;
-	float4 box = s.fat[leafShape[sortedLeaf[k]]];
-	nodeBox[node] = box;
-	nodeHeight[node] = 0;
-	if (n == 1)
-	{
-		countersOut[BC_HEIGHT] = 0;
-		return;
-	}
-	int p = parent[node];
-	while (p >= 0)
-	{
-		__threadfence();
-		int arrived = atomicAdd(visit + p, 1);
-		if (arrived == 0)
-		{
-			return; // the sibling subtree finishes this node
-		}
-		int2 ch = children[p];
-		// L2 reads: the sibling published its box before its atomicAdd (threadfence above), L1 may not have it
-		float4 a = __ldcg(nodeBox + ch.x), b = __ldcg(nodeBox + ch.y);
-		box = make_float4(fminf(a.x, b.x), fminf(a.y, b.y), fmaxf(a.z, b.z), fmaxf(a.w, b.w));
-		nodeBox[p] = box;
-		// the two child boxes side by side with their parent: a query reads both with one 32-byte access
-		pairBox[2 * p] = a;
-		pairBox[2 * p + 1] = b;
-		int h = 1 + max(__ldcg(nodeHeight + ch.x), __ldcg(nodeHeight + ch.y));
-		nodeHeight[p] = h;
-		if (p == 0)
-		{
-			countersOut[BC_HEIGHT] = h;
-		}
-		p = parent[p];
+		sortedShape[k] = leafShape[leafOut[k]];
 	}
 }
 
@@ -509,29 +484,36 @@ __device__ __forceinline__ void s2bBlockAppend(bool take, int value, int* list, 
 	}
 }
 
-// The queries of this pass: the sorted-leaf indices of the proxies that moved (BC_MOVED, movedLeaves) — neighbours in Morton
-// order stay neighbours in the list, a warp's queries walk the same part of the tree — except up to S2B_MAX_LARGE_MOVERS
-// proxies with LARGE boxes (a container wall spanning the scene overlaps thousands of leaves: one thread walking them all
-// takes milliseconds), which go to largeShapes (BC_LARGE) and are tested the other way round: every leaf against that short
-// list (s2bFindPairsLarge). One kernel, one atomic per block (round 1: flag array + split + cub select).
+// The queries of this pass are the proxies that moved (BC_MOVED, movedShapes), in Morton order — neighbours stay
+// neighbours in the list, a warp's queries share the nodes they test — except up to S2B_MAX_LARGE_MOVERS proxies with
+// LARGE boxes (a container wall spanning the scene overlaps thousands of leaves: one thread testing them all takes
+// milliseconds), which go to largeShapes (BC_LARGE) and are tested the other way round: every leaf against that short
+// list (s2bFindPairsLarge). "Large" is measured against the scene box of the last rebuild.
 #define S2B_MAX_LARGE_MOVERS 64
 
-__global__ void s2bCollectMovers(ShapeView s, const int* leafShape, const int* sortedLeaf, int* counters, const float4* nodeBox, int* movedLeaves,
-								 int* largeShapes)
+// Refit of the hierarchy and collection of the queries in one launch (256 threads a block). Thread k copies the box of
+// sorted leaf k; the 16-lane groups reduce level 1, each block reduces its level-2 node, and the last block to finish
+// reduces the levels above. The pass clears BC_REFIT_DONE before this runs.
+__global__ void __launch_bounds__(256) s2bRefit(ShapeView s, const int* sortedShape, int* counters, const int* boundsBits,
+												 float4* nodeBox, int* movedShapes, int* largeShapes)
 {
 	int n = counters[BC_LEAVES];
+	int nh = n - min(counters[BC_LARGE_LEAVES], S2B_MAX_LARGE_LEAVES);
 	int k = blockIdx.x * blockDim.x + threadIdx.x;
 	bool moved = false;
+	int shape = -1;
+	float4 box = s2bEmptyBox();
 	if (k < n)
 	{
-		int shape = leafShape[sortedLeaf[k]];
+		shape = sortedShape[k];
+		box = s.fat[shape];
+		nodeBox[k] = box;
 		moved = (s.head[shape].x & S2B_SHAPE_MOVED) != 0;
 		if (moved && n >= 256)
 		{
-			float4 root = nodeBox[0];
-			float4 box = s.fat[shape];
+			float sceneArea = (s2bOrderedToFloat(boundsBits[6]) - s2bOrderedToFloat(boundsBits[4])) *
+							  (s2bOrderedToFloat(boundsBits[7]) - s2bOrderedToFloat(boundsBits[5]));
 			float area = (box.z - box.x) * (box.w - box.y);
-			float sceneArea = (root.z - root.x) * (root.w - root.y);
 			if (area * 256.0f > sceneArea)
 			{
 				int slot = atomicAdd(counters + BC_LARGE, 1);
@@ -543,7 +525,61 @@ __global__ void s2bCollectMovers(ShapeView s, const int* leafShape, const int* s
 			}
 		}
 	}
-	s2bBlockAppend(moved, k, movedLeaves, counters + BC_MOVED);
+	s2bBlockAppend(moved, shape, movedShapes, counters + BC_MOVED);
+
+	int offset[S2B_MAX_LEVELS], count[S2B_MAX_LEVELS];
+	int top = s2bLevels(n, nh, offset, count);
+	__shared__ float4 level1[256 / S2B_FANOUT];
+	__shared__ bool lastBlock;
+	float4 group = s2bUnion16(k < nh ? box : s2bEmptyBox());
+	if ((threadIdx.x & (S2B_FANOUT - 1)) == 0)
+	{
+		if (top >= 1 && k < nh)
+		{
+			nodeBox[offset[1] + k / S2B_FANOUT] = group;
+		}
+		level1[threadIdx.x / S2B_FANOUT] = group;
+	}
+	__syncthreads();
+	if (threadIdx.x < 32)
+	{
+		float4 node = s2bUnion16(threadIdx.x < 256 / S2B_FANOUT ? level1[threadIdx.x] : s2bEmptyBox());
+		if (threadIdx.x == 0 && top >= 2 && blockIdx.x * 256 < nh)
+		{
+			nodeBox[offset[2] + blockIdx.x] = node;
+		}
+	}
+	if (threadIdx.x == 0)
+	{
+		__threadfence();
+		lastBlock = atomicAdd(counters + BC_REFIT_DONE, 1) == (int)gridDim.x - 1;
+	}
+	__syncthreads();
+	if (lastBlock == false)
+	{
+		return;
+	}
+	__threadfence();
+	for (int l = 3; l <= top; ++l)
+	{
+		const float4* below = nodeBox + offset[l - 1];
+		for (int i = threadIdx.x; i < count[l]; i += blockDim.x)
+		{
+			int first = i * S2B_FANOUT, last = min(first + S2B_FANOUT, count[l - 1]);
+			float4 r = s2bEmptyBox();
+			for (int j = first; j < last; ++j)
+			{
+				// L2 reads: level 2 was written by the other blocks
+				r = s2bUnion(r, __ldcg(below + j));
+			}
+			nodeBox[offset[l] + i] = r;
+		}
+		__syncthreads();
+	}
+	if (threadIdx.x == 0)
+	{
+		counters[BC_HEIGHT] = top + 1;
+	}
 }
 
 // what the query of proxy Q does with an overlapping proxy `other` (reference s2PairQueryCallback, src/broad_phase.c:166-258)
@@ -653,91 +689,125 @@ __device__ __forceinline__ bool s2bMakeQuery(PairQuery& q, int shapeQ, const Sha
 
 #define S2B_QUERY_BATCH 16
 
-// moved proxies with ordinary boxes: one thread walks the hierarchy
-__global__ void __launch_bounds__(128) s2bFindPairs(ShapeView s, BodyView b, const int* leafShape, const int* sortedLeaf, int* counters,
-								 const int* movedLeaves, const int2* children, const float4* pairBox,
-								 const unsigned long long* pairHash, unsigned long long hashMask, const unsigned long long* jointKeys,
-								 int jointKeyCount, unsigned long long* newKey, int2* newShapes, int newCap)
+// bit j set: child box j of the `count` (<= 16) boxes at `boxes` overlaps q; the loads are independent
+__device__ __forceinline__ unsigned s2bOverlapMask(const float4* __restrict__ boxes, int count, float4 q)
 {
+	unsigned mask = 0;
+#pragma unroll
+	for (int j = 0; j < S2B_FANOUT; ++j)
+	{
+		if (j < count && s2bBoxesOverlap(q, __ldg(boxes + j)))
+		{
+			mask |= 1u << j;
+		}
+	}
+	return mask;
+}
+
+// survivors: both shapes alive and not re-created, fat AABBs still overlap (reference src/world.c:149-166), and no joint
+// created since forbids the pair (reference src/joint.c:214-217)
+// The survivors' slots are appended to keepSlots (BC_KEPT): their order does not matter, the merged table is sorted by pair key.
+__device__ __forceinline__ void s2bCollectKeptContacts(int i, const ContactView& c, int contactCount, const ShapeView& s,
+														const unsigned long long* jointKeys, int jointKeyCount, int* keepSlots, int* counters)
+{
+	bool keep = false;
+	if (i < contactCount)
+	{
+		int2 sh = c.shapes[i];
+		int4 ha = s.head[sh.x], hb = s.head[sh.y];
+		bool alive = (ha.x & S2B_ROW_VALID) && (hb.x & S2B_ROW_VALID) && (ha.x & S2B_SHAPE_FRESH) == 0 && (hb.x & S2B_SHAPE_FRESH) == 0;
+		keep = alive && s2bBoxesOverlap(s.fat[sh.x], s.fat[sh.y]) && s2bJointOverride(jointKeys, jointKeyCount, ha.y, hb.y) == false;
+	}
+	s2bBlockAppend(keep, i, keepSlots, counters + BC_KEPT);
+}
+
+// Blocks [0, queryBlocks): one thread per moved proxy with an ordinary box walks the hierarchy and tests the large-leaf
+// list. The blocks behind them collect the survivors of the current table, which is independent of the queries and runs in
+// the shadow of their tail.
+__global__ void __launch_bounds__(128) s2bFindPairs(ShapeView s, BodyView b, const int* sortedShape, int* counters, const int* movedShapes,
+													const float4* __restrict__ nodeBox, int queryBlocks, ContactView cur, int contactCount,
+													const unsigned long long* destroyKeys, int destroyKeyCount, int* keepSlots,
+													const unsigned long long* pairHash, unsigned long long hashMask,
+													const unsigned long long* jointKeys, int jointKeyCount, unsigned long long* newKey,
+													int2* newShapes, int newCap)
+{
+	if ((int)blockIdx.x >= queryBlocks)
+	{
+		s2bCollectKeptContacts(((int)blockIdx.x - queryBlocks) * blockDim.x + threadIdx.x, cur, contactCount, s, destroyKeys,
+							   destroyKeyCount, keepSlots, counters);
+		return;
+	}
 	int n = counters[BC_LEAVES];
+	int large = min(counters[BC_LARGE_LEAVES], S2B_MAX_LARGE_LEAVES);
+	int nh = n - large;
 	int movedCount = counters[BC_MOVED];
 	int qi = blockIdx.x * blockDim.x + threadIdx.x;
 	if (qi >= movedCount)
 	{
 		return;
 	}
-	int leaf = movedLeaves[qi];
 	PairQuery q;
-	if (s2bMakeQuery(q, leafShape[sortedLeaf[leaf]], s, b) == false || n == 1)
+	if (s2bMakeQuery(q, movedShapes[qi], s, b) == false)
 	{
 		return;
 	}
 	float4 boxQ = s.fat[q.shapeQ];
 
-	// descend into one overlapping child directly and stack the other: half the stack traffic of push-both / pop.
-	// Overlapping LEAVES are only collected during the walk and examined in batches afterwards: the walk (box tests) and the
-	// pair rules (shape header, hash probe, filters) are two different instruction streams, and a warp whose lanes hit
-	// leaves at different moments would otherwise execute both serially for every lane (10 of 32 lanes active, ncu round 1).
-	int stack[64];
-	int found[S2B_QUERY_BATCH];
+	// Depth-first over the levels with one pending child mask per level. Overlapping LEAVES are only collected during the
+	// walk and examined in batches afterwards: the walk (box tests) and the pair rules (shape header, hash probe, filters)
+	// are two different instruction streams, and a warp whose lanes hit leaves at different moments would otherwise
+	// execute both serially for every lane (10 of 32 lanes active, ncu round 1).
+	int offset[S2B_MAX_LEVELS], count[S2B_MAX_LEVELS];
+	int top = s2bLevels(n, nh, offset, count);
+	unsigned pending[S2B_MAX_LEVELS];
+	int base[S2B_MAX_LEVELS];
+	int found[S2B_QUERY_BATCH + S2B_FANOUT];
 	int nFound = 0;
-	int sp = 0;
-	int node = 0;
-	bool walking = true;
+	int level = top;
+	bool walking = nh > 0;
+	if (walking)
+	{
+		pending[top] = s2bOverlapMask(nodeBox + offset[top], count[top], boxQ);
+		base[top] = 0;
+	}
 	while (walking || nFound > 0)
 	{
 		while (walking && nFound < S2B_QUERY_BATCH)
 		{
-			if (node >= n - 1)
+			unsigned m = pending[level];
+			if (level == 0 || m == 0)
 			{
-				found[nFound++] = node - (n - 1);
-				if (sp == 0)
+				for (; m != 0; m &= m - 1)
 				{
-					walking = false;
-					break;
+					found[nFound++] = base[0] + __ffs(m) - 1;
 				}
-				node = stack[--sp];
+				level += 1;
+				walking = level <= top;
 				continue;
 			}
-			int2 ch = children[node];
-			bool o0 = s2bBoxesOverlap(boxQ, pairBox[2 * node]);
-			bool o1 = s2bBoxesOverlap(boxQ, pairBox[2 * node + 1]);
-			if (o0 && o1)
-			{
-				if (sp < 64)
-				{
-					stack[sp++] = ch.y;
-				}
-				node = ch.x;
-			}
-			else if (o0)
-			{
-				node = ch.x;
-			}
-			else if (o1)
-			{
-				node = ch.y;
-			}
-			else
-			{
-				if (sp == 0)
-				{
-					walking = false;
-					break;
-				}
-				node = stack[--sp];
-			}
+			pending[level] = m & (m - 1);
+			int first = (base[level] + __ffs(m) - 1) * S2B_FANOUT;
+			pending[level - 1] = s2bOverlapMask(nodeBox + offset[level - 1] + first, min(S2B_FANOUT, count[level - 1] - first), boxQ);
+			base[level - 1] = first;
+			level -= 1;
 		}
 		for (int k = 0; k < nFound; ++k)
 		{
-			s2bConsiderPair(q, leafShape[sortedLeaf[found[k]]], s, b, counters, pairHash, hashMask, jointKeys, jointKeyCount, newKey, newShapes,
+			s2bConsiderPair(q, sortedShape[found[k]], s, b, counters, pairHash, hashMask, jointKeys, jointKeyCount, newKey, newShapes,
 							newCap);
 		}
 		nFound = 0;
 	}
+	for (int i = nh; i < n; ++i)
+	{
+		if (s2bBoxesOverlap(boxQ, nodeBox[i]))
+		{
+			s2bConsiderPair(q, sortedShape[i], s, b, counters, pairHash, hashMask, jointKeys, jointKeyCount, newKey, newShapes, newCap);
+		}
+	}
 }
 
-// every leaf against the short list of large movers (s2bCollectMovers). Same rules, same pairs; the order new pairs are
+// every leaf against the short list of large movers (s2bRefit). Same rules, same pairs; the order new pairs are
 // emitted in never matters (they are sorted).
 __global__ void s2bFindPairsLarge(ShapeView s, BodyView b, const int* leafShape, int* counters, const int* largeShapes,
 								  const unsigned long long* pairHash, unsigned long long hashMask, const unsigned long long* jointKeys,
@@ -765,24 +835,6 @@ __global__ void s2bFindPairsLarge(ShapeView s, BodyView b, const int* leafShape,
 			s2bConsiderPair(q, other, s, b, counters, pairHash, hashMask, jointKeys, jointKeyCount, newKey, newShapes, newCap);
 		}
 	}
-}
-
-// survivors: both shapes alive and not re-created, fat AABBs still overlap (reference src/world.c:149-166), and no joint
-// created since forbids the pair (reference src/joint.c:214-217)
-// The survivors' slots are appended to keepSlots (BC_KEPT): their order does not matter, the merged table is sorted by pair key.
-__global__ void s2bCollectKeptContacts(ContactView c, int contactCount, ShapeView s, const unsigned long long* jointKeys, int jointKeyCount,
-									   int* keepSlots, int* counters)
-{
-	int i = blockIdx.x * blockDim.x + threadIdx.x;
-	bool keep = false;
-	if (i < contactCount)
-	{
-		int2 sh = c.shapes[i];
-		int4 ha = s.head[sh.x], hb = s.head[sh.y];
-		bool alive = (ha.x & S2B_ROW_VALID) && (hb.x & S2B_ROW_VALID) && (ha.x & S2B_SHAPE_FRESH) == 0 && (hb.x & S2B_SHAPE_FRESH) == 0;
-		keep = alive && s2bBoxesOverlap(s.fat[sh.x], s.fat[sh.y]) && s2bJointOverride(jointKeys, jointKeyCount, ha.y, hb.y) == false;
-	}
-	s2bBlockAppend(keep, i, keepSlots, counters + BC_KEPT);
 }
 
 // The sort key is the pair key squeezed to 2 x shapeBits bits (lo << shapeBits | hi) so the radix sort runs only over
@@ -910,15 +962,11 @@ static size_t bpReserve(s2bWorld* w, BroadScratch* B)
 	B->mortonOut.reserve(nS, st, false);
 	B->leafIn.reserve(nS, st, false);
 	B->leafOut.reserve(nS, st, false);
+	B->sortedShape.reserve(nS, st, false);
 	B->counters.reserve(BC_SIZE, st, false);
-	B->boundsBits.reserve(4, st, false);
-	B->children.reserve(nS, st, false);
-	B->parent.reserve(2 * nS, st, false);
-	B->nodeBox.reserve(2 * nS, st, false);
-	B->pairBox.reserve(2 * nS, st, false);
-	B->visit.reserve(nS, st, false);
-	B->nodeHeight.reserve(2 * nS, st, false);
-	B->movedLeaves.reserve(nS, st, false);
+	B->boundsBits.reserve(8, st, false);
+	B->nodeBox.reserve(nS + nS / 8 + 64, st, false); // leaves + levels: n (1 + 1/16 + 1/256 + ...) + one per level
+	B->movedShapes.reserve(nS, st, false);
 	B->movedFlag.reserve(nS, st, false);
 	B->largeShapes.reserve(S2B_MAX_LARGE_MOVERS, st, false);
 	B->keepFlag.reserve((size_t)std::max(oldCount, 1), st, false);
@@ -940,7 +988,7 @@ static size_t bpReserve(s2bWorld* w, BroadScratch* B)
 	return tempBytes;
 }
 
-// First half of a pass, no host synchronisation: hierarchy (re-used or rebuilt) and refit, pair-key hash of the current
+// First half of a pass, no host synchronisation: sorted order (re-used or rebuilt) and refit, pair-key hash of the current
 // table, queries from the moved proxies -> candidate pairs (newKey / newShapes), survivors of the current table (keepSlots),
 // and the counters of all that copied to the pinned mailbox.
 static void bpSearch(s2bWorld* w, BroadScratch* B)
@@ -951,13 +999,14 @@ static void bpSearch(s2bWorld* w, BroadScratch* B)
 	ShapeView sv = shapeView(w);
 	BodyView bv = bodyView(w);
 	ContactColumns& cur = w->contacts[w->cur];
-	size_t nS = (size_t)shapeCap;
 	int newCap = B->newPairCap;
 
+	// the sorted order (and with it the hierarchy's topology and the large-leaf list) is reused while no shape was
+	// created, destroyed or re-uploaded; boxes drift a little per step, a periodic re-sort keeps the nodes tight
 	bool reuseTree = B->treeValid && w->pairsDirty == false && B->treeShapeCap == shapeCap && B->treeReuses < S2B_TREE_REUSE_LIMIT;
 	if (reuseTree)
 	{
-		// keep BC_LEAVES (and the stale height); clear the per-pass counters
+		// keep BC_LEAVES / BC_LARGE_LEAVES; clear the per-pass counters
 		S2B_CHECK(cudaMemsetAsync(B->counters.p + BC_NEW_PAIRS, 0, sizeof(int) * (BC_SIZE - BC_NEW_PAIRS), st));
 		B->treeReuses += 1;
 	}
@@ -972,9 +1021,10 @@ static void bpSearch(s2bWorld* w, BroadScratch* B)
 								   B->counters.p + BC_LEAVES, shapeCap, st);
 		w->kernelLaunches += 2;
 
-		// ---- Morton order ----
-		int initBounds[4] = {0x7F7FFFFF, 0x7F7FFFFF, (int)0x80800000, (int)0x80800000};
+		// ---- Morton order, large leaves last ----
 		// ordered encoding: +FLT_MAX -> 0x7F7FFFFF, -FLT_MAX -> 0xFF7FFFFF ^ 0x7FFFFFFF = 0x80800000
+		const int lo = 0x7F7FFFFF, hi = (int)0x80800000;
+		int initBounds[8] = {lo, lo, hi, hi, lo, lo, hi, hi};
 		S2B_CHECK(cudaMemcpyAsync(B->boundsBits.p, initBounds, sizeof(initBounds), cudaMemcpyHostToDevice, st));
 		S2B_LAUNCH(w, s2bSceneBounds, gridFor(shapeCap, 256), 256, 0, sv, B->leafShape.p, B->counters.p, B->boundsBits.p);
 		S2B_LAUNCH(w, s2bMortonCodes, gridFor(shapeCap, 256), 256, 0, sv, B->leafShape.p, B->counters.p, B->boundsBits.p,
@@ -982,18 +1032,16 @@ static void bpSearch(s2bWorld* w, BroadScratch* B)
 		tb = B->cubTemp.cap;
 		cub::DeviceRadixSort::SortPairs(B->cubTemp.p, tb, B->mortonIn.p, B->mortonOut.p, B->leafIn.p, B->leafOut.p, shapeCap, 0, 32, st);
 		w->kernelLaunches += 5;
-
-		// ---- hierarchy ----
-		S2B_LAUNCH(w, s2bBuildRadixTree, gridFor(shapeCap, 256), 256, 0, B->mortonOut.p, B->counters.p, B->children.p, B->parent.p);
+		S2B_LAUNCH(w, s2bSortedShapes, gridFor(shapeCap, 256), 256, 0, B->leafShape.p, B->leafOut.p, B->counters.p, B->sortedShape.p);
 		B->treeValid = true;
 		B->treeShapeCap = shapeCap;
 		B->treeReuses = 0;
+		w->pairRebuildCount += 1;
 	}
 
-	// ---- refit ----
-	S2B_CHECK(cudaMemsetAsync(B->visit.p, 0, sizeof(int) * nS, st));
-	S2B_LAUNCH(w, s2bRefit, gridFor(shapeCap, 256), 256, 0, sv, B->leafShape.p, B->leafOut.p, B->counters.p, B->children.p,
-			   B->parent.p, B->nodeBox.p, B->pairBox.p, B->visit.p, B->nodeHeight.p, B->counters.p);
+	// ---- refit, and the moved proxies ----
+	S2B_LAUNCH(w, s2bRefit, gridFor(shapeCap, 256), 256, 0, sv, B->sortedShape.p, B->counters.p, B->boundsBits.p, B->nodeBox.p,
+			   B->movedShapes.p, B->largeShapes.p);
 
 	// ---- pair-key hash set of the current contact table (rebuilt only when the table changed) ----
 	if (B->hashVersion != w->contactTableVersion || B->pairHash.p == nullptr)
@@ -1013,21 +1061,14 @@ static void bpSearch(s2bWorld* w, BroadScratch* B)
 		B->hashVersion = w->contactTableVersion;
 	}
 
-	// ---- queries from moved proxies ----
-	S2B_LAUNCH(w, s2bCollectMovers, gridFor(shapeCap, 256), 256, 0, sv, B->leafShape.p, B->leafOut.p, B->counters.p, B->nodeBox.p,
-			   B->movedLeaves.p, B->largeShapes.p);
-	S2B_LAUNCH(w, s2bFindPairs, gridFor(shapeCap, 128), 128, 0, sv, bv, B->leafShape.p, B->leafOut.p, B->counters.p,
-			   B->movedLeaves.p, B->children.p, B->pairBox.p, B->pairHash.p, B->hashMask, w->jointPairKeys.p, w->jointPairCount,
-			   B->newKey.p, B->newShapes.p, newCap);
+	// ---- queries from moved proxies, and the survivors ----
+	int queryBlocks = gridFor(shapeCap, 128);
+	S2B_LAUNCH(w, s2bFindPairs, queryBlocks + (oldCount > 0 ? gridFor(oldCount, 128) : 0), 128, 0, sv, bv, B->sortedShape.p,
+			   B->counters.p, B->movedShapes.p, B->nodeBox.p, queryBlocks, makeView(cur), oldCount, w->jointDestroyKeys.p,
+			   w->jointDestroyCount, B->keepSlots.p, B->pairHash.p, B->hashMask, w->jointPairKeys.p, w->jointPairCount, B->newKey.p,
+			   B->newShapes.p, newCap);
 	S2B_LAUNCH(w, s2bFindPairsLarge, gridFor(shapeCap, 256), 256, 0, sv, bv, B->leafShape.p, B->counters.p, B->largeShapes.p,
 			   B->pairHash.p, B->hashMask, w->jointPairKeys.p, w->jointPairCount, B->newKey.p, B->newShapes.p, newCap);
-
-	// ---- survivors ----
-	if (oldCount > 0)
-	{
-		S2B_LAUNCH(w, s2bCollectKeptContacts, gridFor(oldCount, 256), 256, 0, makeView(cur), oldCount, sv, w->jointDestroyKeys.p,
-				   w->jointDestroyCount, B->keepSlots.p, B->counters.p);
-	}
 	S2B_CHECK(cudaMemcpyAsync(w->hostMail + MAIL_BC_BASE, B->counters.p, sizeof(int) * BC_SIZE, cudaMemcpyDeviceToHost, st));
 	B->searchedCount = oldCount;
 	B->searchedVersion = w->contactTableVersion;
@@ -1167,6 +1208,7 @@ void s2bBroadphaseUpdatePairs(s2bWorld* w)
 			if (fresh <= B->newPairCap)
 			{
 				w->treeHeight = hc[BC_HEIGHT];
+				w->largeLeafCount = std::min(hc[BC_LARGE_LEAVES], S2B_MAX_LARGE_LEAVES);
 				B->lastPassRan = hc[BC_MOVED] > 0 || hc[BC_LARGE] > 0;
 				bpCommit(w, B, fresh, kept, B->prefetchTempBytes);
 				return;
@@ -1215,6 +1257,7 @@ void s2bBroadphaseUpdatePairs(s2bWorld* w)
 			continue; // rare: redo the pass with a larger pair buffer
 		}
 		w->treeHeight = hc[BC_HEIGHT];
+		w->largeLeafCount = std::min(hc[BC_LARGE_LEAVES], S2B_MAX_LARGE_LEAVES);
 		bpCommit(w, B, fresh, kept, tempBytes);
 		break;
 	}

@@ -376,6 +376,8 @@ struct s2bWorld
 	DevArray<int> dMovedFlag; // [0] = number of proxies moved in last finalize (device counter)
 	int pairPassCount = 0;
 	int treeHeight = 0;
+	int largeLeafCount = 0;
+	int pairRebuildCount = 0;
 
 	// solve-order hint (validation)
 	std::vector<unsigned long long> orderHint;

@@ -3650,6 +3650,8 @@ extern "C" void s2b_get_counters(s2bWorld* w, s2bCounters* out)
 		}
 	}
 	out->treeHeight = w->treeHeight;
+	out->largeLeafCount = w->largeLeafCount;
+	out->pairRebuildCount = w->pairRebuildCount;
 	out->movedCount = w->hostMail[MAIL_MOVED];
 	out->pairPassCount = w->pairPassCount;
 	out->kernelLaunches = w->kernelLaunches;

@@ -58,7 +58,8 @@ class Counters(C.Structure):
                 ("groupCount", C.c_int32), ("overflowCount", C.c_int32), ("treeHeight", C.c_int32),
                 ("movedCount", C.c_int32), ("pairPassCount", C.c_int32), ("kernelLaunches", C.c_int32),
                 ("graphReplays", C.c_int32), ("graphCaptures", C.c_int32), ("scratchBytes", C.c_int64),
-                ("regionCount", C.c_int32), ("cutCount", C.c_int32), ("cutGroupCount", C.c_int32), ("recolouredCount", C.c_int32)]
+                ("regionCount", C.c_int32), ("cutCount", C.c_int32), ("cutGroupCount", C.c_int32), ("recolouredCount", C.c_int32),
+                ("largeLeafCount", C.c_int32), ("pairRebuildCount", C.c_int32)]
 
 
 SCHEDULE_COLOR, SCHEDULE_WAVEFRONT = 0, 1
